@@ -1,6 +1,7 @@
 """Headline benchmark: pose estimates / second at num_envs=1024 (BASELINE.json), one process per GPU.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--num-envs 1024] [--precision fp16f8|fp16x2|bf16x3|bf16]
+                    [--dump-outputs DIR]
 
 A step = one pass of the hot path (preprocess -> backbone x2 views -> plane-sweep volume -> 3-D U-Net -> decode ->
 fit) over ALL num_envs environments of synthetic input.  With N > 1 (torchrun) the environments are sharded
@@ -19,6 +20,9 @@ stays num_envs, i.e. strong scaling, as the metric is defined at num_envs=1024.
            observation + actor step of the N=4096 / 8-GPU configuration as this rank's share) -- reported beside the headline.
 `--impl reference`: the reference's own CPU implementation (oracle/_ref: a run-time copy of the unmodified reference staged
            by __graft_entry__.build(); the oracle port if that copy is absent) timed on the host cores on a bounded sample.
+`--dump-outputs DIR`: after the timed steps, the boxes of the last timed step (what estimate() hands its caller, all num_envs
+           environments) go to DIR/boxes.npy as float64.  Inputs, weights and the per-call sampler seeds depend only on the
+           arguments, so two builds run with the same arguments can be compared box for box.
 """
 from __future__ import annotations
 
@@ -57,6 +61,7 @@ CFG = {"name": "adapose_v5", "task_name": "one_drawer_cabinet", "load": False, "
        "n_pts": 1024, "direct_regression": True, "real_world": False}
 DEFAULT_BBOX = np.asarray([[0, 0, 0], [0, 0, 1], [0, 1, 0], [0, 1, 1], [1, 0, 0], [1, 0, 1], [1, 1, 0], [1, 1, 1]], dtype=np.float64) + 10.0
 TOL_PX, TOL_DEG, TOL_MM = 0.5, 0.5, 1.0
+DUMP_MAX_BYTES = 64 << 20
 
 
 def workload_name(n):
@@ -109,6 +114,18 @@ class ClockSampler:
                 pass
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": mx or None, "reasons": sorted(reasons),
                 "samples": len(sm)}
+
+
+def dump_output(out_dir, name, t):
+    """Write one output as out_dir/<name>.npy.  Beyond DUMP_MAX_BYTES only a fixed, seeded sample of its rows (environments),
+    in ascending order, is written, so that the file stays comparable between runs with the same arguments."""
+    a = t.cpu().numpy()
+    row = max(1, a[:1].nbytes)
+    keep = (DUMP_MAX_BYTES - 4096) // row          # 4 KB for the .npy header
+    if len(a) > keep:
+        a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def dist_setup():
@@ -336,7 +353,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU legs (profiling runs)")
     ap.add_argument("--no-extra", action="store_true", help="skip the other BASELINE configurations and the e2e variants")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the boxes of the last timed step to DIR/boxes.npy (float64 [num_envs, 8, 3]; a seeded sample of the "
+                         "environments if that exceeds 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl in ("reference", "cpu-sample"):
+        ap.error("--dump-outputs writes the outputs of the device path, not of the CPU reference arm")
     if args.impl in ("reference", "cpu-sample"):
         os.environ["CUDA_VISIBLE_DEVICES"] = ""         # the CPU arm must not see a GPU (see cpu_legs_subprocess); set before CUDA initialises
     if args.impl == "cpu-sample":
@@ -382,8 +406,11 @@ def main():
         dist.all_gather_into_tensor(gathered, pad)
         return gathered[:N]
 
+    last = {}
+
     def step_device():
-        return gather(est.estimate(*[devt[k] for k in order], return_tensor=True, env_offset=lo))
+        last["boxes"] = gather(est.estimate(*[devt[k] for k in order], return_tensor=True, env_offset=lo))
+        return last["boxes"]
 
     def step_host(src=host):
         return gather(est.estimate(*[src[k] for k in order], return_tensor=True, env_offset=lo)).cpu()
@@ -424,6 +451,8 @@ def main():
     clocks = sampler.stop()
     value = N * args.steps / (ms / 1e3)
     eng.check_error_flag()
+    if args.dump_outputs and rank == 0:
+        dump_output(args.dump_outputs, "boxes", last["boxes"])     # before the next gather reuses its buffer
 
     e2e = None
     h2d = sum(host[k].numel() * host[k].element_size() for k in order)
