@@ -6,7 +6,6 @@
 
 #include "../../include/adapose_b200.h"
 #include "common.cuh"
-#include <stdlib.h>
 #include "tc_conv.cuh"
 
 namespace adp {
@@ -160,14 +159,11 @@ int adp_conv_tc_plan(adp_conv_plan** plan, const adp_act* in, const void* w_hi, 
     }
     p.out_cs = ep->out_cstride ? ep->out_cstride : cout; p.out_coff = ep->out_coff; p.bias_per_batch = ep->bias_per_batch;
     p.check_finite = ep->check_finite;
-    {
-        // coalesced epilogue stores need full accumulator chunks (bf16 hi + lo planes, fp32 / fp16 side outputs are fine)
-        const int ch = pl->layer.BN < 32 ? pl->layer.BN : 32;
-        static const bool off = getenv("ADP_NO_COALESCE") != nullptr;
-        p.coalesce = (!off && (!ep->out_lo || !in->f16) && cout % ch == 0 && ((cout | p.out_cs | p.out_coff) & 7) == 0) ? 1 : 0;
-    }
+    // coalesced epilogue stores need full accumulator chunks (bf16 hi + lo planes, fp32 / fp16 side outputs are fine)
+    const int ch = pl->layer.BN < 32 ? pl->layer.BN : 32;
+    p.coalesce = ((!ep->out_lo || !in->f16) && cout % ch == 0 && ((cout | p.out_cs | p.out_coff) & 7) == 0) ? 1 : 0;
     pl->num_sms = num_sms > 0 ? num_sms : 148;
-    r = tc_conv_finish_epilogue(&pl->layer);
+    r = tc_conv_finish_plan(&pl->layer);
     if (r != ADP_OK) {
         delete pl;
         return r;

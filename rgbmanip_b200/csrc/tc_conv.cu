@@ -324,7 +324,7 @@ constexpr int kTcThreads = 192;   // warp 0: TMA producer, warp 1: MMA issuer + 
 //            producer's fp8 twin; W8 = e4m3(W_lo 2^16); 128 channels per stage, K = 32 per MMA), then the fp16 sweep with
 //            [A | W_hi] stages whose first MMA scales the accumulator by 2^-15 (scale-input-d).  1.5 MMA passes per
 //            algorithmic FLOP instead of 2, same stage size (48 KB at BN = 256: 4 stages instead of 2).
-template <int BN, int KC, int FUSED = 0, bool NCAT_EN = false>
+template <int BN, int KC, int FUSED = 0>
 struct TcCfg {
     static constexpr int A_BYTES = 128 * KC * 2;
     static constexpr int B_BYTES = BN * KC * 2;
@@ -333,27 +333,20 @@ struct TcCfg {
     static constexpr int STAGE_BYTES = FUSED == 1 ? 2 * (A_BYTES + B_PAD) : FUSED == 2 ? (A_BYTES + 2 * B_PAD) : (A_BYTES + B_PAD);
     // small-N layers are latency bound per tile: fewer stages -> several CTAs per SM overlap their pipelines
     static constexpr int CTAS_PER_SM = FUSED ? ((BN <= 64 && FUSED != 3) ? 2 : 1) : (BN <= 16 && KC <= 32) ? 5 : BN <= 32 ? 3 : (BN <= 64 ? 2 : 1);
-    // fp16x2 with a narrow N tile: W_hi and W_lo sit back to back in the stage, so ONE MMA of N = 2 BN reads the A operand once
-    // and leaves A W_hi in columns [0, BN) and A W_lo in [BN, 2 BN) of the accumulator; the epilogue adds the two halves.  A
-    // BN <= 64 MMA is bound by the 128 B/clk shared-memory operand path (4 KB of A per MMA), not by the tensor pipe: reading A
-    // once instead of twice takes a K step from 12 KB to 8 KB of operand traffic at the same tensor work.  The epilogue reads
-    // twice the accumulator columns, so this pays only for layers with a long K loop (>= 18 K steps per tile: up_2 0.96 ->
-    // 0.86 ms per 148 frames; the 9-step layers layer1 / up_3 are epilogue bound and lose 5-10 %): tc_conv_plan decides.
-    static constexpr bool NCAT = NCAT_EN && FUSED == 2 && BN <= 64 && (B_BYTES % 1024 == 0);
     static constexpr int EPI_BYTES = 4 * 2048;                  // per-epilogue-warp transpose buffers (coalesced stores)
     static constexpr int SMEM_BUDGET = (220 * 1024 - CTAS_PER_SM * (EPI_BYTES + 2048)) / CTAS_PER_SM;
     static constexpr int STAGES = (STAGE_BYTES * 6 <= SMEM_BUDGET) ? 6 : (SMEM_BUDGET / STAGE_BYTES);
-    static constexpr int ACC_STRIDE = NCAT ? 2 * BN : (BN < 32 ? 32 : BN);   // TMEM columns per accumulator stage
+    static constexpr int ACC_STRIDE = BN < 32 ? 32 : BN;   // TMEM columns per accumulator stage
     static constexpr int TMEM_COLS = (2 * ACC_STRIDE <= 64) ? 64 : (2 * ACC_STRIDE <= 128) ? 128 : (2 * ACC_STRIDE <= 256) ? 256 : 512;
     static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + EPI_BYTES + 1024 /*align slack*/ + 256 /*barriers*/;
 };
 
-template <int BN, int KC, int FUSED, bool NCAT_EN>
-__global__ void __launch_bounds__(kTcThreads, TcCfg<BN, KC, FUSED, NCAT_EN>::CTAS_PER_SM)
+template <int BN, int KC, int FUSED>
+__global__ void __launch_bounds__(kTcThreads, TcCfg<BN, KC, FUSED>::CTAS_PER_SM)
 tc_conv_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
                const __grid_constant__ CUtensorMap tmW_hi, const __grid_constant__ CUtensorMap tmW_lo,
                const TcConvParams p, int batch) {
-    using Cfg = TcCfg<BN, KC, FUSED, NCAT_EN>;
+    using Cfg = TcCfg<BN, KC, FUSED>;
     constexpr int STAGES = Cfg::STAGES;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -472,7 +465,7 @@ tc_conv_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
         uint32_t phase = 0;
         int as = 0;
         uint32_t aphase = 0;
-        const uint32_t idesc = make_idesc<Cfg::NCAT ? 2 * BN : BN>(p.f16);
+        const uint32_t idesc = make_idesc<BN>(p.f16);
         const uint32_t elected = ptx::elect_one();
         const uint32_t tbase = __shfl_sync(0xffffffffu, tmem_base, 0);
         for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
@@ -483,13 +476,7 @@ tc_conv_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
                 ptx::mbar_wait(full_bar(stage), phase, p.err, 3);
                 ptx::tc_fence_after();
                 const uint32_t sa = smem_base + stage * Cfg::STAGE_BYTES;
-                if (FUSED == 2 && Cfg::NCAT) {
-                    const uint64_t ah = make_smem_desc<KC>(sa);
-                    const uint64_t whl = make_smem_desc<KC>(sa + Cfg::A_BYTES);      // rows [0, BN) = W_hi, [BN, 2 BN) = W_lo
-#pragma unroll
-                    for (int k = 0; k < KC / 16; ++k)
-                        ptx::umma_bf16_elected(tmem_d, ah + (uint64_t)(2 * k), whl + (uint64_t)(2 * k), idesc, (it > 0 || k > 0) ? 1u : 0u, elected);
-                } else if (FUSED == 2) {
+                if (FUSED == 2) {
                     const uint64_t ah = make_smem_desc<KC>(sa);
                     const uint64_t wh = make_smem_desc<KC>(sa + Cfg::A_BYTES);
                     const uint64_t wl = make_smem_desc<KC>(sa + Cfg::A_BYTES + Cfg::B_PAD);
@@ -577,16 +564,6 @@ tc_conv_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
                 const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(as * Cfg::ACC_STRIDE + c0);
                 ptx::tmem_ld16(taddr, r);
                 if (CH == 32) ptx::tmem_ld16(taddr + 16, r + 16);
-                if (Cfg::NCAT) {          // accumulator columns [BN, 2 BN) hold the W_lo products of the same outputs
-                    uint32_t r2[16];
-#pragma unroll
-                    for (int h = 0; h < CH / 16; ++h) {
-                        ptx::tmem_ld16(taddr + BN + 16 * h, r2);
-                        ptx::tmem_ld_wait();
-#pragma unroll
-                        for (int j = 0; j < 16; ++j) r[16 * h + j] = __float_as_uint(__uint_as_float(r[16 * h + j]) + __uint_as_float(r2[j]));
-                    }
-                }
                 ptx::tmem_ld_wait();
                 const int nbase = n0 + c0;
                 if (nbase < p.Cout) {       // Cout may be padded up to BN (e.g. 8 -> 16); uniform over the warp
@@ -910,7 +887,6 @@ slab_conv_kernel(const __grid_constant__ CUtensorMap tmSlab, const __grid_consta
 // host side
 // ------------------------------------------------------------------------------------------------
 static PFN_cuTensorMapEncodeTiled_v12000 g_encode = nullptr;
-static int g_fuse_max_bn = -1;   // split-precision layers with BN <= this share hi/lo stages (ADP_FUSE_MAXBN overrides)
 PFN_cuTensorMapEncodeTiled_v12000 g_encode_shared = nullptr;   // for the other tcgen05 translation units
 
 int tc_conv_init_driver() {
@@ -1036,16 +1012,10 @@ int tc_conv_plan(TcConvLayer* L, const Act& in, const bf16* w_hi, const bf16* w_
     p.npass = npass;
     L->BN = BN;
     L->KC = KC;
-    if (g_fuse_max_bn < 0) {
-        const char* e = getenv("ADP_FUSE_MAXBN");
-        g_fuse_max_bn = e ? atoi(e) : 256;
-    }
-    L->fused = (npass >= 2) && (BN <= g_fuse_max_bn) && KC >= 16;
-    ADP_CHECK_ARG(npass != 4 || (BN == 256 || BN == 128 || BN == 64), "fp16 + fp8 low-order pass: Cout tile of 64, 128 or 256");
+    ADP_CHECK_ARG(npass != 4 || BN == 256 || BN == 128, "the fp8 low-order pass needs a Cout tile of 128 or 256");
     // slab mode: single K chunk, single pass, small N, unit strides, a tap window of at most 3 planes x 4 x 4, 8 | W
-    L->slab = false;
+    L->slab_ctas = 0;
     {
-        static const bool off = getenv("ADP_NO_SLAB") != nullptr;
         int lo[3] = {127, 127, 127}, hi[3] = {-127, -127, -127};
         for (int t = 0; t < p.ntaps; ++t) {
             const int o[3] = {p.tdz[t], p.tdy[t], p.tdx[t]};
@@ -1053,7 +1023,7 @@ int tc_conv_plan(TcConvLayer* L, const Act& in, const bf16* w_hi, const bf16* w_
         }
         const bool shape_ok = (BN == 16 && (KC == 16 || KC == 64)) || (BN == 64 && KC == 16) || (BN == 32 && KC == 32);
         // (2-D maps qualify too: the s2d stem runs here as 2 x 16 taps - hi and lo weight slabs of the same 4 x 4 window)
-        if (!off && p.kchunks == 1 && npass == 1 && coutPad == BN && shape_ok && p.in_mul == 1 && p.out_mul == 1 &&
+        if (p.kchunks == 1 && npass == 1 && coutPad == BN && shape_ok && p.in_mul == 1 && p.out_mul == 1 &&
             p.out_oz == 0 && p.out_oy == 0 && p.out_ox == 0 && p.W % 8 == 0 && p.ntaps >= 4 &&
             hi[0] - lo[0] <= 2 && hi[1] - lo[1] <= 3 && hi[2] - lo[2] <= 3) {
             p.TW = 8; p.TH = 16;
@@ -1064,12 +1034,9 @@ int tc_conv_plan(TcConvLayer* L, const Act& in, const bf16* w_hi, const bf16* w_
             const int stage_bytes = (p.slab_bytes + 1023) & ~1023;
             const int w_slot = (BN * KC * 2 + 1023) / 1024 * 1024;
             const int fixed = p.ntaps * w_slot + 8192 + 1024 + 512;
-            int ctas = 2;                                             // CTAs per SM (see tc_conv_launch)
+            // CTAs per SM; 32 -> 32 channels (conv4: 35 KB slabs + 54 KB of weights) runs one CTA per SM with more stages
+            const int ctas = (BN == 32 && KC == 32) ? 1 : 2;
             int stages = (220 * 1024 / ctas - fixed) / stage_bytes;
-            if (stages < 2 && BN == 32 && KC == 32) {                 // conv4 (32 -> 32, 35 KB slabs + 54 KB of weights): one CTA per SM
-                ctas = 1;
-                stages = (220 * 1024 - fixed) / stage_bytes;
-            }
             stages = stages > 6 ? 6 : stages;
             if (stages >= 2) {
                 p.slab_stages = stages;
@@ -1086,7 +1053,6 @@ int tc_conv_plan(TcConvLayer* L, const Act& in, const bf16* w_hi, const bf16* w_
                     set_last_error("cuTensorMapEncodeTiled(slab %dx%dx%d x %d) failed: %d", p.sSX, p.sSY, p.sSZ, KC, (int)r);
                     return ADP_ERR_CUDA;
                 }
-                L->slab = true;
             } else {
                 tc_pick_tile(p.H, p.W, &p.TW, &p.TH);
                 p.tiles_x = cdiv(p.W, p.TW); p.tiles_y = cdiv(p.H, p.TH);
@@ -1102,15 +1068,15 @@ int tc_conv_plan(TcConvLayer* L, const Act& in, const bf16* w_hi, const bf16* w_
         ADP_TRY(encode_act_map(&L->tmA_lo, in.lo ? in.lo : in.hi, in, KC, p.TW, p.TH, p.in_mul, f16));
         ADP_TRY(encode_w_map(&L->tmW_lo, w_lo ? w_lo : w_hi, in.C, coutPad, w_taps, KC, BN, f16));
     }
-    L->ready = true;
     return ADP_OK;
 }
 
-int tc_conv_finish_epilogue(TcConvLayer* L) {
+// after the epilogue fields of L->p are set: the TMA epilogue where it applies, and its tensor maps
+static int tc_conv_pick_bulk_epilogue(TcConvLayer* L) {
     TcConvParams& p = L->p;
     L->bulk_epi = false;
     const bool off = getenv("ADP_NO_BULK_EPI") != nullptr;        // read per plan: the A/B test builds one engine each way
-    if (off || !L->slab || L->BN != 64 || L->KC != 16 || p.Cout != 64 || !p.f16 || !p.coalesce) return ADP_OK;
+    if (off || !L->slab_ctas || L->BN != 64 || L->KC != 16 || p.Cout != 64 || !p.f16 || !p.coalesce) return ADP_OK;
     if (!p.res_hi || p.res_lo || p.res_cs != 64 || !p.out_hi || p.out_lo || p.out_cs != 64 || p.out_coff != 0) return ADP_OK;
     if (p.out_f32 || p.out_h16 || p.out_q8 || p.bias_per_batch || p.TW != 8 || p.TH != 16) return ADP_OK;
     if (((uintptr_t)p.res_hi | (uintptr_t)p.out_hi) & 15) return ADP_OK;
@@ -1140,17 +1106,17 @@ int tc_conv_finish_epilogue(TcConvLayer* L) {
     return ADP_OK;
 }
 
-template <int BN, int KC, int FUSED = 0, bool NCAT_EN = false>
+template <int BN, int KC, int FUSED = 0>
 static int launch_impl(const TcConvLayer* L, int batch, int num_sms, cudaStream_t stream) {
-    using Cfg = TcCfg<BN, KC, FUSED, NCAT_EN>;
+    using Cfg = TcCfg<BN, KC, FUSED>;
     static int attr[kMaxDevices];
-    ADP_TRY(ensure_dyn_smem(tc_conv_kernel<BN, KC, FUSED, NCAT_EN>, Cfg::SMEM_BYTES, attr));
+    ADP_TRY(ensure_dyn_smem(tc_conv_kernel<BN, KC, FUSED>, Cfg::SMEM_BYTES, attr));
     const TcConvParams& p = L->p;
     long long total = (long long)batch * p.D * p.tiles_y * p.tiles_x * p.tiles_n;
     const long long slots = (long long)num_sms * Cfg::CTAS_PER_SM;
     int grid = (int)(total < slots ? total : slots);
     if (grid <= 0) return ADP_OK;
-    tc_conv_kernel<BN, KC, FUSED, NCAT_EN><<<grid, kTcThreads, Cfg::SMEM_BYTES, stream>>>(L->tmA_hi, L->tmA_lo, L->tmW_hi, L->tmW_lo, p, batch);
+    tc_conv_kernel<BN, KC, FUSED><<<grid, kTcThreads, Cfg::SMEM_BYTES, stream>>>(L->tmA_hi, L->tmA_lo, L->tmW_hi, L->tmW_lo, p, batch);
     ADP_CUDA(cudaGetLastError());
     return ADP_OK;
 }
@@ -1173,48 +1139,68 @@ static int launch_slab(const TcConvLayer* L, int batch, int num_sms, cudaStream_
     return ADP_OK;
 }
 
+// Every kernel instance there is.  slab_ctas 0: the generic kernel; FUSED 0 = one pass, or the pass loop of split precision,
+// 1 = bf16x3, 2 = fp16x2, 3 = fp16 + fp8 low-order pass.  slab_ctas > 0: the slab kernel (single pass) for that many CTAs per SM,
+// bulk = TMA epilogue.
+struct TcInstance {
+    int slab_ctas;
+    bool bulk;
+    int fused, BN, KC;
+    decltype(TcConvLayer::launch) launch;
+};
+static const TcInstance kTcInstances[] = {
+    {0, false, 0, 256, 64, launch_impl<256, 64>},
+    {0, false, 0, 128, 64, launch_impl<128, 64>},
+    {0, false, 0, 64, 64, launch_impl<64, 64>},
+    {0, false, 0, 32, 64, launch_impl<32, 64>},
+    {0, false, 0, 16, 64, launch_impl<16, 64>},
+    {0, false, 0, 64, 32, launch_impl<64, 32>},
+    {0, false, 0, 32, 16, launch_impl<32, 16>},
+    {0, false, 1, 256, 64, launch_impl<256, 64, 1>},
+    {0, false, 1, 128, 64, launch_impl<128, 64, 1>},
+    {0, false, 1, 64, 64, launch_impl<64, 64, 1>},
+    {0, false, 1, 32, 64, launch_impl<32, 64, 1>},
+    {0, false, 1, 64, 16, launch_impl<64, 16, 1>},
+    {0, false, 2, 256, 64, launch_impl<256, 64, 2>},
+    {0, false, 2, 128, 64, launch_impl<128, 64, 2>},
+    {0, false, 2, 64, 64, launch_impl<64, 64, 2>},
+    {0, false, 2, 32, 64, launch_impl<32, 64, 2>},
+    {0, false, 3, 256, 64, launch_impl<256, 64, 3>},
+    {0, false, 3, 128, 64, launch_impl<128, 64, 3>},
+    {2, false, 0, 16, 16, launch_slab<16, 16, 2>},
+    {2, false, 0, 16, 64, launch_slab<16, 64, 2>},
+    {2, false, 0, 64, 16, launch_slab<64, 16, 2>},         // (3 CTAs per SM spill: 1.5 -> 1.9 ms)
+    {2, true, 0, 64, 16, launch_slab<64, 16, 2, true>},
+    {1, false, 0, 32, 32, launch_slab<32, 32, 1>},
+};
+
+static decltype(TcConvLayer::launch) find_instance(int slab_ctas, bool bulk, int fused, int BN, int KC) {
+    for (const TcInstance& t : kTcInstances)
+        if (t.slab_ctas == slab_ctas && t.bulk == bulk && t.fused == fused && t.BN == BN && t.KC == KC) return t.launch;
+    return nullptr;
+}
+
+int tc_conv_finish_plan(TcConvLayer* L) {
+    ADP_TRY(tc_conv_pick_bulk_epilogue(L));
+    // split precision keeps its hi and lo operands in one pipeline stage where (BN, KC) has such an instance, and otherwise runs
+    // the passes one after another through the FUSED = 0 kernel (the narrow per-point MLP layers)
+    const int npass = L->p.npass;
+    const int fused = npass == 2 ? 2 : npass == 3 ? 1 : npass == 4 ? 3 : 0;
+    L->launch = find_instance(L->slab_ctas, L->bulk_epi, fused, L->BN, L->KC);
+    if (!L->launch && (npass == 2 || npass == 3)) L->launch = find_instance(0, false, 0, L->BN, L->KC);
+    if (!L->launch) {
+        static const char* const mode[] = {"", "single pass", "fp16x2", "bf16x3", "fp16 + fp8 low-order pass"};
+        set_last_error("no tcgen05 conv instantiation for BN=%d KC=%d (%s%s)", L->BN, L->KC, mode[npass],
+                       L->slab_ctas ? ", slab kernel" : "");
+        return ADP_ERR_ARG;
+    }
+    return ADP_OK;
+}
+
 int tc_conv_launch(const TcConvLayer* L, int batch, int num_sms, cudaStream_t stream) {
-    ADP_CHECK_ARG(L->ready, "layer not planned");
+    ADP_CHECK_ARG(L->launch, "layer not planned");
     ADP_CHECK_ARG(batch <= L->p.B, "batch exceeds planned capacity");
-    if (L->slab) {
-        if (L->BN == 16 && L->KC == 16) return launch_slab<16, 16, 2>(L, batch, num_sms, stream);
-        if (L->BN == 16 && L->KC == 64) return launch_slab<16, 64, 2>(L, batch, num_sms, stream);
-        if (L->BN == 64 && L->KC == 16 && L->bulk_epi) return launch_slab<64, 16, 2, true>(L, batch, num_sms, stream);
-        if (L->BN == 64 && L->KC == 16) return launch_slab<64, 16, 2>(L, batch, num_sms, stream);   // (3 CTAs per SM spill: 1.5 -> 1.9 ms)
-        if (L->BN == 32 && L->KC == 32 && L->slab_ctas == 1) return launch_slab<32, 32, 1>(L, batch, num_sms, stream);
-        if (L->BN == 32 && L->KC == 32) return launch_slab<32, 32, 2>(L, batch, num_sms, stream);
-        set_last_error("no slab conv instantiation for BN=%d KC=%d", L->BN, L->KC);
-        return ADP_ERR_ARG;
-    }
-    if (L->p.npass == 3 && L->fused) {   // bf16x3: one stage carries hi and lo operands
-        if (L->BN == 64 && L->KC == 64) return launch_impl<64, 64, 1>(L, batch, num_sms, stream);
-        if (L->BN == 32 && L->KC == 64) return launch_impl<32, 64, 1>(L, batch, num_sms, stream);
-        if (L->BN == 64 && L->KC == 16) return launch_impl<64, 16, 1>(L, batch, num_sms, stream);
-        if (L->BN == 128 && L->KC == 64) return launch_impl<128, 64, 1>(L, batch, num_sms, stream);
-        if (L->BN == 256 && L->KC == 64) return launch_impl<256, 64, 1>(L, batch, num_sms, stream);
-    }
-    if (L->p.npass == 4) {               // fp16 pass + fp8 low-order pass
-        if (L->BN == 256 && L->KC == 64) return launch_impl<256, 64, 3>(L, batch, num_sms, stream);
-        if (L->BN == 128 && L->KC == 64) return launch_impl<128, 64, 3>(L, batch, num_sms, stream);
-        if (L->BN == 64 && L->KC == 64) return launch_impl<64, 64, 3>(L, batch, num_sms, stream);
-        set_last_error("no fp16 + fp8lo instantiation for BN=%d KC=%d", L->BN, L->KC);
-        return ADP_ERR_ARG;
-    }
-    if (L->p.npass == 2 && L->fused) {   // fp16x2: one stage carries A, W_hi, W_lo
-        if (L->BN == 64 && L->KC == 64 && L->p.ntaps * L->p.kchunks >= 18) return launch_impl<64, 64, 2, true>(L, batch, num_sms, stream);
-        if (L->BN == 64 && L->KC == 64) return launch_impl<64, 64, 2>(L, batch, num_sms, stream);
-        if (L->BN == 32 && L->KC == 64) return launch_impl<32, 64, 2>(L, batch, num_sms, stream);
-        if (L->BN == 64 && L->KC == 16) return launch_impl<64, 16, 2>(L, batch, num_sms, stream);
-        if (L->BN == 128 && L->KC == 64) return launch_impl<128, 64, 2>(L, batch, num_sms, stream);
-        if (L->BN == 256 && L->KC == 64) return launch_impl<256, 64, 2>(L, batch, num_sms, stream);
-    }
-#define ADP_TC_CASE(bn, kc) if (L->BN == bn && L->KC == kc) return launch_impl<bn, kc>(L, batch, num_sms, stream)
-    ADP_TC_CASE(256, 64); ADP_TC_CASE(128, 64); ADP_TC_CASE(64, 64); ADP_TC_CASE(32, 64); ADP_TC_CASE(16, 64);
-    ADP_TC_CASE(64, 32); ADP_TC_CASE(32, 32); ADP_TC_CASE(16, 32);
-    ADP_TC_CASE(64, 16); ADP_TC_CASE(32, 16); ADP_TC_CASE(16, 16);
-#undef ADP_TC_CASE
-    set_last_error("no tcgen05 conv instantiation for BN=%d KC=%d", L->BN, L->KC);
-    return ADP_ERR_ARG;
+    return L->launch(L, batch, num_sms, stream);
 }
 
 }  // namespace adp

@@ -64,14 +64,14 @@ struct TcConvLayer {
     TcConvParams p;
     int BN;
     int KC;                  // channels per K step (64 -> SWIZZLE_128B, 32 -> 64B, 16 -> 32B)
-    bool fused = false;      // split precision with hi and lo operands sharing a pipeline stage
-    bool slab = false;       // one halo slab per tile, taps by descriptor offsets, weights resident (slab_conv_kernel)
+    int slab_ctas = 0;       // > 0: slab mode (one halo slab per tile, taps by descriptor offsets, weights resident:
+                             // slab_conv_kernel), with stages sized for this many CTAs per SM
     CUtensorMap tmSlab;
-    int slab_ctas = 2;       // CTAs per SM the slab stages were sized for
     bool bulk_epi = false;   // slab mode, 64 fp16 channels in and out with a 64-channel residual: residual tiles arrive by TMA, results
-                             // leave by TMA store (tc_conv_finish_epilogue decides)
+                             // leave by TMA store (tc_conv_finish_plan decides)
     CUtensorMap tmRes, tmOut;
-    bool ready = false;
+    // the kernel instance of this layer, chosen by tc_conv_finish_plan; null until the plan is complete
+    int (*launch)(const TcConvLayer* L, int batch, int num_sms, cudaStream_t stream) = nullptr;
 };
 
 int tc_conv_init_driver();
@@ -87,8 +87,9 @@ struct TcGeom {             // non-standard geometries (NULL = stride-1 "same" c
 
 int tc_conv_plan(TcConvLayer* L, const Act& in, const bf16* w_hi, const bf16* w_lo, int Cout, int kd, int ks,
                  int dil, int npass, const TcGeom* geom, int f16);
-// after the epilogue fields of L->p are set: picks the TMA epilogue where it applies and encodes its tensor maps
-int tc_conv_finish_epilogue(TcConvLayer* L);
+// after the epilogue fields of L->p are set: picks the TMA epilogue where it applies and the kernel instance; ADP_ERR_ARG when
+// the library has no instance for the layer's tile, K step and pass mode
+int tc_conv_finish_plan(TcConvLayer* L);
 int tc_conv_launch(const TcConvLayer* L, int batch, int num_sms, cudaStream_t stream);
 
 }  // namespace adp

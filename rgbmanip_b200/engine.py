@@ -60,10 +60,17 @@ class ActBuf:
         return v if n is None else v[:n]
 
 
-def _split_bf16(w: torch.Tensor):
-    hi = w.to(torch.bfloat16)
-    lo = (w - hi.float()).to(torch.bfloat16)
-    return hi, lo
+def pack_tc_weights(wt: torch.Tensor, f16: int, npass: int):
+    """fp32 [taps, CoutPad, Cin] weights -> the (hi, lo) planes adp_conv_tc_plan reads, on the host.  bf16: hi + lo split (lo for
+    bf16x3 only); fp16: hi, plus the fp16 rounding residual as lo for fp16x2 (npass 2), or as e4m3(W_lo * 2^16) bytes for the fp8
+    low-order pass (npass 4, see tc_conv.cu FUSED = 3).  lo is None for a single pass."""
+    hi = wt.to(torch.float16 if f16 else torch.bfloat16)
+    lo = wt - hi.float()
+    if npass == 1:
+        return hi, None
+    if npass == 4:
+        return hi, (lo * 65536.0).clamp(-448.0, 448.0).to(torch.float8_e4m3fn).view(torch.uint8)
+    return hi, lo.to(hi.dtype)
 
 
 class Engine:
@@ -168,22 +175,13 @@ class Engine:
 
     def _tc_plans(self, x: ActBuf, wt, cout, kd, ks, dil, npass, ep, geoms):
         """wt: fp32 [taps, CoutPad, Cin] packed weights -> callable(batch) launching one tcgen05 conv per geometry."""
-        if x.f16:
-            hi, lo = wt.to(torch.float16), None
-            if npass == 2:
-                lo = (wt - hi.float()).to(torch.float16).to(self.device).contiguous()
-            elif npass == 4:     # low-order term for the fp8 pass: e4m3(W_lo * 2^16), one byte per weight (see tc_conv.cu FUSED = 3)
-                lo = ((wt - hi.float()) * 65536.0).clamp(-448.0, 448.0).to(torch.float8_e4m3fn).view(torch.uint8).to(self.device).contiguous()
-        else:
-            hi, lo = _split_bf16(wt)
-            lo = lo.to(self.device).contiguous()
-        hi = hi.to(self.device).contiguous()
+        hi, lo = (t.to(self.device).contiguous() if t is not None else None for t in pack_tc_weights(wt, x.f16, npass))
         self._keep += [hi, lo]
         plans = []
         xa = x.c
         for g in geoms:
             plan = C.c_void_p()
-            L.check(self.lib.adp_conv_tc_plan(C.byref(plan), C.byref(xa), L.ptr(hi), L.ptr(lo) if npass >= 2 else None,
+            L.check(self.lib.adp_conv_tc_plan(C.byref(plan), C.byref(xa), L.ptr(hi), L.ptr(lo),
                                               cout, kd, ks, dil, npass, C.byref(ep), C.byref(g) if g is not None else None,
                                               self.num_sms), "conv_tc_plan")
             self._plans.append(plan)
@@ -194,6 +192,11 @@ class Engine:
                 L.check(self.lib.adp_conv_tc_run(plan, batch, L.ptr(self.err_flag), self.stream), "conv_tc_run")
         run.kind = "tc"
         return run
+
+    def _with_fp8lo(self, npass, x: ActBuf, plain=True):
+        """fp16f8: an fp16x2 conv (npass 2) runs its low-order term as the fp8 pass (npass 4) when x carries an fp8 twin, Cin is a
+        multiple of 128 and the conv is plain (2-D, stride 1, not transposed)."""
+        return 4 if (npass == 2 and self.fp8lo and plain and x.q8 is not None and x.Cn % 128 == 0) else npass
 
     def _conv(self, w_np, x: ActBuf, out: ActBuf | None, *, stride=1, dil=1, transposed=False, npass=None, **ep_kw):
         """Returns a callable(batch) running the convolution x -> out.  w_np: torch layout
@@ -209,9 +212,7 @@ class Engine:
         kd = w.shape[2] if three_d else 1
         ks = w.shape[-1]
         assert cin == x.Cn
-        npass = self.npass if npass is None else npass
-        if npass == 2 and self.fp8lo and x.q8 is not None and cin % 128 == 0 and not three_d and stride == 1 and not transposed:
-            npass = 4
+        npass = self._with_fp8lo(self.npass if npass is None else npass, x, plain=not three_d and stride == 1 and not transposed)
         can_tc = (cin % 16 == 0 and ks in (1, 3) and (ks == w.shape[-2]) and stride in (1, 2)
                   and (npass == 1 or (npass in (2, 4) and x.f16) or (npass == 3 and x.lo is not None)))
         ep = self._epilogue(out, **ep_kw)
@@ -253,11 +254,9 @@ class Engine:
         ops.append(("pack_s2d", lambda b, o=s2d: L.check(
             self.lib.adp_pack_s2d(L.ptr(self.crops), C.byref(o.c), b, S, self.stream), "pack_s2d")))
         wst = G.stem_s2d_weights(w)
-        if s2d.f16 and self.npass == 2 and S % 32 == 0:
+        if s2d.f16 and self.npass == 2:
             # fp16 hi + lo weights as 2 x 16 taps of a single pass on the slab kernel (geometry.stem_s2d_split)
-            w_hi = wst.to(torch.float16).float()
-            w_lo = (wst - w_hi).to(torch.float16).float()
-            ops.append(("conv1", self._tc_plans(s2d, torch.cat([w_hi, w_lo], 0), 64, 1, 4, 1, 1,
+            ops.append(("conv1", self._tc_plans(s2d, torch.cat(pack_tc_weights(wst, 1, 2)).float(), 64, 1, 4, 1, 1,
                                                 self._epilogue(c1, act=L.ACT_RELU), [G.stem_s2d_split(S)])))
         else:
             ops.append(("conv1", self._tc_plans(s2d, wst, 64, 1, 4, 1, self.npass,
@@ -322,7 +321,7 @@ class Engine:
             if nm in restructured:
                 wt = wgt.permute(2, 3, 0, 1).reshape(1, 9 * cout, wgt.shape[1]).contiguous()      # [1][(ky*3+kx)*Cout + co][Cin]
                 q = self._act(F, x.H, x.W, 9 * cout)
-                npass = 4 if (self.npass == 2 and self.fp8lo and x.q8 is not None and x.Cn % 128 == 0) else self.npass
+                npass = self._with_fp8lo(self.npass, x)
                 gemm = self._tc_plans(x, wt, 9 * cout, 1, 1, 1, npass, self._epilogue(q, act=L.ACT_NONE), [None])
                 ops.append((f"{nm}.taps", gemm))
 

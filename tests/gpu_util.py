@@ -67,6 +67,7 @@ def tc_conv(x_cl, w, *, dil=1, npass=3, bias=None, scale=None, act_code=L.ACT_NO
     """x_cl: fp32 [B,(D,)H,W,Cin] cpu; w: torch layout [Cout,Cin,(kd,)k,k] ([Cin,Cout,3,3,3] when transposed).
     Returns (fp32 output, 16-bit output as fp32), cpu, channels-last."""
     from rgbmanip_b200 import geometry
+    from rgbmanip_b200.engine import pack_tc_weights
     lib = L.load()
     three_d = x_cl.dim() == 5
     B = x_cl.shape[0]
@@ -92,22 +93,16 @@ def tc_conv(x_cl, w, *, dil=1, npass=3, bias=None, scale=None, act_code=L.ACT_NO
     cpad = (Cout + 15) // 16 * 16
     if cpad != Cout:
         wt = torch.cat([wt, torch.zeros(wt.shape[0], cpad - Cout, Cin)], 1).contiguous()
+    wh, wl = (t.to(DEV).contiguous() if t is not None else None for t in pack_tc_weights(wt, f16, npass))
+    xq = None
     if f16:
         xh, xl = x_cl.to(torch.float16).to(DEV).contiguous(), None
-        wh16 = wt.to(torch.float16)
-        wh, wl = wh16.to(DEV).contiguous(), None
-        xq = None
-        if npass == 2:      # fp16x2: the rounding residual of the weights rides in a second fp16 plane
-            wl = (wt - wh16.float()).to(torch.float16).to(DEV).contiguous()
-        elif npass == 4:    # fp16 + fp8 low-order pass: e4m3(W_lo 2^16) against the activation's e4m3(x / 2) twin
-            wl = to_e4m3((wt - wh16.float()) * 65536.0).to(DEV).contiguous()
+        if npass == 4:      # the activation's e4m3(x / 2) twin for the fp8 low-order pass
             xq = to_e4m3(x_cl.to(torch.float16).float() * 0.5).to(DEV).contiguous()
         dt16 = torch.float16
     else:
         xh, xl = split(x_cl, npass == 3)
-        wh, wl = split(wt, npass == 3)
         dt16 = torch.bfloat16
-        xq = None
     out_f32 = torch.full(oshape, float("nan"), dtype=torch.float32, device=DEV)
     out_hi = torch.zeros(out_f32.shape, dtype=dt16, device=DEV)
     out_lo = torch.zeros_like(out_hi) if not f16 else None

@@ -47,7 +47,7 @@ TC2D_CASES = [
     (1, 224, 224, 64, 64, 3, 1),
     (1, 224, 224, 64, 32, 1, 1),
     (3, 20, 12, 64, 128, 3, 1),
-    (2, 20, 24, 64, 64, 3, 1),          # fp16x2: slab kernel with [W_hi | W_lo] slots, partial tiles in y
+    (2, 20, 24, 64, 64, 3, 1),          # 24 x 5 pixel tiles: 8 of the 128 MMA rows stay unused
 ]
 
 
@@ -93,7 +93,7 @@ FP8LO_CASES = [
     (1, 28, 28, 128, 256, 1, 1),
     (3, 28, 28, 512, 512, 3, 4),
     (1, 56, 56, 1024, 256, 3, 1),
-    (1, 20, 12, 128, 64, 3, 1),
+    (1, 20, 12, 128, 128, 3, 1),
 ]
 
 
@@ -126,11 +126,11 @@ def test_tc_conv2d_fp16_plus_fp8_low_order_pass(G, case):
 
 TC3D_CASES = [
     # (B, D, H, W, Cin, Cout)
-    (1, 6, 28, 28, 32, 8),
+    (1, 6, 28, 28, 64, 8),
     (1, 5, 56, 56, 16, 16),
-    (2, 6, 28, 28, 32, 32),
+    (2, 6, 28, 56, 32, 32),
     (1, 3, 28, 28, 64, 64),
-    (1, 4, 224, 224, 32, 8),
+    (1, 4, 224, 224, 64, 8),
 ]
 
 
@@ -155,10 +155,10 @@ TC_GEOM_CASES = [
     (3, 1, 6, 56, 56, 32, 64, 3, 2, False, 1),
     (3, 1, 6, 56, 56, 32, 64, 3, 2, False, 0),
     (3, 1, 3, 28, 28, 64, 32, 3, 2, True, 1),
-    (3, 1, 6, 56, 56, 32, 16, 3, 2, True, 1),
-    (3, 2, 4, 28, 28, 16, 8, 3, 2, True, 1),
-    (3, 1, 4, 28, 28, 16, 8, 3, 2, True, 0),
-    (3, 1, 5, 56, 56, 32, 8, 3, 1, False, 1),
+    (3, 1, 6, 56, 56, 64, 16, 3, 2, True, 1),
+    (3, 2, 4, 28, 28, 64, 8, 3, 2, True, 1),
+    (3, 1, 4, 28, 28, 64, 8, 3, 2, True, 0),
+    (3, 1, 5, 56, 56, 64, 8, 3, 1, False, 1),
 ]
 
 
@@ -192,6 +192,24 @@ def test_tc_conv_strided_transposed_fp16(G, case):
     assert torch.isfinite(out32).all()
     assert G.rel_err(G.from_cl(out32), ref) < 1e-4        # operands exactly representable: fp32 summation order only
     assert G.rel_err(G.from_cl(out16), ref) < (2e-3 if f16 else 1.2e-2)   # 16-bit output rounding
+
+
+def test_tc_conv_plan_rejects_a_layer_without_kernel_instance(G):
+    """A layer whose tile (BN x KC) and pass mode have no kernel instance fails when it is planned, not at its first launch:
+    a stride-2 3-D conv from 32 to 8 channels needs BN 16 x KC 32 in a single pass, which no layer of the network uses."""
+    from rgbmanip_b200 import geometry
+    lib = L.load()
+    B, D, H, W, Cin, Cout = 1, 4, 28, 28, 32, 8
+    x = torch.zeros((B, D, H, W, Cin), dtype=torch.float16, device=G.DEV)
+    w = torch.zeros((27, 16, Cin), dtype=torch.float16, device=G.DEV)
+    out = torch.zeros((B, D // 2, H // 2, W // 2, Cout), dtype=torch.float16, device=G.DEV)
+    ep = G.epilogue(out_hi=out)
+    a = G.act(x, None, B, D, H, W, Cin, 1)
+    plan = C.c_void_p()
+    with pytest.raises(L.AdpError, match=r"BN=16 KC=32 \(single pass\)"):
+        L.check(lib.adp_conv_tc_plan(C.byref(plan), C.byref(a), L.ptr(w), None, Cout, 3, 3, 1, 1, C.byref(ep),
+                                     C.byref(geometry.strided(True, D, H, W, 3, 2)), 148), "plan")
+    assert plan.value is None
 
 
 @pytest.mark.parametrize("f16", [1, 0])
@@ -370,7 +388,7 @@ def test_maxpool_psp_upsample(G):
     assert G.rel_err(G.from_cl(G.val(zh, zl).cpu()), ref) < 5e-5
 
 
-@pytest.mark.parametrize("case", [(2, 12, 20, 32, 64, 1), (1, 28, 28, 64, 16, 1), (2, 7, 9, 32, 8, 0), (1, 5, 30, 16, 64, 0)],
+@pytest.mark.parametrize("case", [(2, 12, 20, 32, 64, 1), (1, 28, 28, 64, 16, 1), (2, 7, 9, 64, 8, 0), (1, 5, 30, 16, 64, 0)],
                          ids=lambda c: "x".join(map(str, c)))
 def test_upconv_restructured_matches_oracle(G, case):
     """PSPUpsample (pspnet.py:97-107) as per-tap 1x1 GEMM at low resolution (adp_conv_tc) + adp_upconv_blend against
