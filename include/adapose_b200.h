@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define ADP_ABI_VERSION 5
+#define ADP_ABI_VERSION 6
 
 #if defined(__GNUC__)
 #define ADP_API __attribute__((visibility("default")))
@@ -80,7 +80,8 @@ typedef struct adp_epilogue { /* y = act(scale * acc + bias [+ res]) [+ res]  ->
     int32_t out_cstride;      /* channel pitch of out_hi/out_lo (0 = Cout): lets a layer write a column range of a wider tensor */
     int32_t out_coff;         /* first channel of that range (torch.cat of network_v5.py:488 without a copy) */
     int32_t bias_per_batch;   /* 1: bias is [B, Cout] (the per-env global feature term of pose_mlp2, network_v5.py:491-493) */
-    void* out_q8;             /* optional fp8 (e4m3) twin of out_hi holding value / 2 (same channel pitch / offset), or NULL: see adp_act.q8 */
+    void* out_q8;             /* optional fp8 (e4m3) twin of out_hi holding value / 2 (same channel pitch / offset), or NULL: see adp_act.q8;
+                                 needs fp16, Cout % 32 == 0 and out_cstride, out_coff multiples of 16 (else ADP_ERR_ARG at plan time) */
     int32_t check_finite;     /* 1: OR bit 0 into err_flag[1] when an output value is inf/NaN (fp16 range guard, set on the last backbone layer) */
 } adp_epilogue;
 
@@ -122,6 +123,15 @@ ADP_API int adp_conv_tc_plan(adp_conv_plan** plan, const adp_act* in, const void
 /* err_flag: int32[2] on the device -- [0] pipeline watchdog code (a stuck barrier traps the kernel instead of hanging the GPU),
  * [1] range flag (see adp_epilogue.check_finite).  The same two-word flag is passed to every *_run entry point. */
 ADP_API int adp_conv_tc_run(adp_conv_plan* plan, int batch, int32_t* err_flag, void* stream);
+/* The kernel instance a plan chose and its tiling, read-only (tests use it to tie each reference case to an instance).
+ * info: int32[ADP_TC_PLAN_INFO_LEN] =
+ *   [0] row of the instance table (tc_conv.cu kTcInstances)   [1] slab CTAs per SM (0: generic kernel)   [2] TMA epilogue
+ *   [3] FUSED: 0 single pass or the split-precision pass loop, 1 bf16x3, 2 fp16x2, 3 fp16 + fp8 low-order pass
+ *   [4] BN   [5] KC   [6] npass of the layer   [7] TW   [8] TH   [9] coalesced epilogue stores
+ *   [10] tiles_x   [11] tiles_y   [12] tiles_n   [13] tile-grid depth (tiles per image = [10] [11] [12] [13])
+ *   [14] K chunks   [15] taps */
+#define ADP_TC_PLAN_INFO_LEN 16
+ADP_API int adp_conv_tc_plan_info(const adp_conv_plan* plan, int32_t* info);
 ADP_API void adp_conv_tc_free(adp_conv_plan* plan);
 ADP_API int adp_maxpool3x3s2(const adp_act* in, const adp_act* out, int batch, void* stream);                 /* pspnet.py:39 */
 /* feat_cstride: channel pitch of feat (0 = dense); the engine lets layer4's last conv write straight into the first 512

@@ -8,10 +8,11 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "libadapose_b200.so")
 
-ADP_ABI_VERSION = 5
+ADP_ABI_VERSION = 6
 DT_U8, DT_F32, DT_F64 = 0, 1, 2
 ACT_NONE, ACT_RELU, ACT_PRELU, ACT_TANH = 0, 1, 2, 3
 LAYOUT_F16, LAYOUT_S2D = 1, 2          # adp_decode x11_format / adp_conv0_plan_create flags
+TC_PLAN_INFO_LEN = 16                  # int32 fields of adp_conv_tc_plan_info
 
 vp = C.c_void_p
 i32 = C.c_int32
@@ -59,6 +60,7 @@ SIGNATURES = {
     "adp_conv_tc_plan": (C.c_int, [C.POINTER(vp), C.POINTER(Act), vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                    C.POINTER(Epilogue), C.POINTER(TcGeom), C.c_int]),
     "adp_conv_tc_run": (C.c_int, [vp, C.c_int, vp, vp]),
+    "adp_conv_tc_plan_info": (C.c_int, [vp, vp]),
     "adp_conv_tc_free": (None, [vp]),
     "adp_maxpool3x3s2": (C.c_int, [C.POINTER(Act), C.POINTER(Act), C.c_int, vp]),
     "adp_psp_priors": (C.c_int, [C.POINTER(Act), C.c_int, vp, vp, vp, C.c_int, vp]),

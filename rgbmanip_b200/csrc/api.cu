@@ -162,6 +162,14 @@ int adp_conv_tc_plan(adp_conv_plan** plan, const adp_act* in, const void* w_hi, 
     // coalesced epilogue stores need full accumulator chunks (bf16 hi + lo planes, fp32 / fp16 side outputs are fine)
     const int ch = pl->layer.BN < 32 ? pl->layer.BN : 32;
     p.coalesce = ((!ep->out_lo || !in->f16) && cout % ch == 0 && ((cout | p.out_cs | p.out_coff) & 7) == 0) ? 1 : 0;
+    // only the coalesced stores write the fp8 twin, in 16-byte row pieces (one byte per channel): a layer whose twin would stay
+    // unwritten, or whose pieces would be misaligned, fails here instead of leaving stale bytes for the consumer's low-order pass
+    if (p.out_q8 && (!p.coalesce || ((p.out_cs | p.out_coff) & 15) || ((uintptr_t)ep->out_q8 & 15))) {
+        set_last_error("out_q8 is written by the coalesced epilogue only, in 16-byte pieces: out_cstride (%d) and out_coff (%d) must be "
+                       "multiples of 16 and the plane 16-byte aligned", p.out_cs, p.out_coff);
+        delete pl;
+        return ADP_ERR_ARG;
+    }
     pl->num_sms = num_sms > 0 ? num_sms : 148;
     r = tc_conv_finish_plan(&pl->layer);
     if (r != ADP_OK) {
@@ -177,6 +185,11 @@ int adp_conv_tc_run(adp_conv_plan* plan, int batch, int32_t* err_flag, void* str
     plan->layer.p.err = err_flag;
     g_launches += 1;
     return tc_conv_launch(&plan->layer, batch, plan->num_sms, (cudaStream_t)stream);
+}
+
+int adp_conv_tc_plan_info(const adp_conv_plan* plan, int32_t* info) {
+    ADP_CHECK_ARG(plan && info, "null pointer");
+    return tc_conv_plan_info(&plan->layer, info);
 }
 
 void adp_conv_tc_free(adp_conv_plan* plan) { delete plan; }

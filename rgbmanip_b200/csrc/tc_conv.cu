@@ -1141,7 +1141,8 @@ static int launch_slab(const TcConvLayer* L, int batch, int num_sms, cudaStream_
 
 // Every kernel instance there is.  slab_ctas 0: the generic kernel; FUSED 0 = one pass, or the pass loop of split precision,
 // 1 = bf16x3, 2 = fp16x2, 3 = fp16 + fp8 low-order pass.  slab_ctas > 0: the slab kernel (single pass) for that many CTAs per SM,
-// bulk = TMA epilogue.
+// bulk = TMA epilogue.  adp_conv_tc_plan_info reports a layer's row by its index: tests/test_gpu_tc_conv.py keeps one reference
+// case per row the engine plans.
 struct TcInstance {
     int slab_ctas;
     bool bulk;
@@ -1174,10 +1175,14 @@ static const TcInstance kTcInstances[] = {
     {1, false, 0, 32, 32, launch_slab<32, 32, 1>},
 };
 
-static decltype(TcConvLayer::launch) find_instance(int slab_ctas, bool bulk, int fused, int BN, int KC) {
-    for (const TcInstance& t : kTcInstances)
-        if (t.slab_ctas == slab_ctas && t.bulk == bulk && t.fused == fused && t.BN == BN && t.KC == KC) return t.launch;
-    return nullptr;
+static constexpr int kTcInstanceCount = (int)(sizeof(kTcInstances) / sizeof(kTcInstances[0]));
+
+static int find_instance(int slab_ctas, bool bulk, int fused, int BN, int KC) {
+    for (int i = 0; i < kTcInstanceCount; ++i) {
+        const TcInstance& t = kTcInstances[i];
+        if (t.slab_ctas == slab_ctas && t.bulk == bulk && t.fused == fused && t.BN == BN && t.KC == KC) return i;
+    }
+    return -1;
 }
 
 int tc_conv_finish_plan(TcConvLayer* L) {
@@ -1186,14 +1191,25 @@ int tc_conv_finish_plan(TcConvLayer* L) {
     // the passes one after another through the FUSED = 0 kernel (the narrow per-point MLP layers)
     const int npass = L->p.npass;
     const int fused = npass == 2 ? 2 : npass == 3 ? 1 : npass == 4 ? 3 : 0;
-    L->launch = find_instance(L->slab_ctas, L->bulk_epi, fused, L->BN, L->KC);
-    if (!L->launch && (npass == 2 || npass == 3)) L->launch = find_instance(0, false, 0, L->BN, L->KC);
-    if (!L->launch) {
+    L->instance = find_instance(L->slab_ctas, L->bulk_epi, fused, L->BN, L->KC);
+    if (L->instance < 0 && (npass == 2 || npass == 3)) L->instance = find_instance(0, false, 0, L->BN, L->KC);
+    if (L->instance < 0) {
         static const char* const mode[] = {"", "single pass", "fp16x2", "bf16x3", "fp16 + fp8 low-order pass"};
         set_last_error("no tcgen05 conv instantiation for BN=%d KC=%d (%s%s)", L->BN, L->KC, mode[npass],
                        L->slab_ctas ? ", slab kernel" : "");
         return ADP_ERR_ARG;
     }
+    L->launch = kTcInstances[L->instance].launch;
+    return ADP_OK;
+}
+
+int tc_conv_plan_info(const TcConvLayer* L, int32_t* info) {
+    ADP_CHECK_ARG(L->instance >= 0 && L->instance < kTcInstanceCount, "layer not planned");
+    const TcInstance& t = kTcInstances[L->instance];
+    const TcConvParams& p = L->p;
+    const int32_t v[16] = {L->instance, t.slab_ctas, t.bulk ? 1 : 0, t.fused, t.BN, t.KC, p.npass, p.TW, p.TH, p.coalesce,
+                           p.tiles_x, p.tiles_y, p.tiles_n, p.D, p.kchunks, p.ntaps};
+    for (int i = 0; i < 16; ++i) info[i] = v[i];
     return ADP_OK;
 }
 

@@ -72,6 +72,7 @@ struct TcConvLayer {
     CUtensorMap tmRes, tmOut;
     // the kernel instance of this layer, chosen by tc_conv_finish_plan; null until the plan is complete
     int (*launch)(const TcConvLayer* L, int batch, int num_sms, cudaStream_t stream) = nullptr;
+    int instance = -1;       // its row in the instance table of tc_conv.cu (reported by tc_conv_plan_info)
 };
 
 int tc_conv_init_driver();
@@ -91,5 +92,7 @@ int tc_conv_plan(TcConvLayer* L, const Act& in, const bf16* w_hi, const bf16* w_
 // the library has no instance for the layer's tile, K step and pass mode
 int tc_conv_finish_plan(TcConvLayer* L);
 int tc_conv_launch(const TcConvLayer* L, int batch, int num_sms, cudaStream_t stream);
+// the chosen instance and tiling of a planned layer: the 16 fields of adp_conv_tc_plan_info (include/adapose_b200.h)
+int tc_conv_plan_info(const TcConvLayer* L, int32_t* info);
 
 }  // namespace adp

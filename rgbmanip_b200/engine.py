@@ -191,6 +191,7 @@ class Engine:
             for plan in plans:
                 L.check(self.lib.adp_conv_tc_run(plan, batch, L.ptr(self.err_flag), self.stream), "conv_tc_run")
         run.kind = "tc"
+        run.plans = plans           # lets a test name the layer behind each plan (adp_conv_tc_plan_info)
         return run
 
     def _with_fp8lo(self, npass, x: ActBuf, plain=True):

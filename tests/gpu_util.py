@@ -52,9 +52,23 @@ def from_cl(x):
 
 
 def epilogue(out_hi=None, out_lo=None, out_f32=None, scale=None, bias=None, act_code=L.ACT_NONE, prelu=0.0, res_hi=None,
-             res_lo=None, res_after_act=0, out_q8=None):
-    return L.Epilogue(L.ptr(scale), L.ptr(bias), float(prelu), act_code, res_after_act, L.ptr(res_hi), L.ptr(res_lo), 0,
-                      L.ptr(out_hi), L.ptr(out_lo), L.ptr(out_f32), None, 0, 0, 0, L.ptr(out_q8), 0)
+             res_lo=None, res_after_act=0, out_q8=None, *, res_cstride=0, out_h16=None, out_cstride=0, out_coff=0, bias_per_batch=0,
+             check_finite=0):
+    """Every field of adp_epilogue (include/adapose_b200.h); tensors may be None."""
+    return L.Epilogue(L.ptr(scale), L.ptr(bias), float(prelu), act_code, res_after_act, L.ptr(res_hi), L.ptr(res_lo), res_cstride,
+                      L.ptr(out_hi), L.ptr(out_lo), L.ptr(out_f32), L.ptr(out_h16), out_cstride, out_coff, bias_per_batch,
+                      L.ptr(out_q8), check_finite)
+
+
+def plan_info(plan):
+    """adp_conv_tc_plan_info as a dict: the kernel instance a plan chose and its tiling."""
+    info = (C.c_int32 * L.TC_PLAN_INFO_LEN)()
+    L.check(L.load().adp_conv_tc_plan_info(plan, info), "plan_info")
+    keys = ("row", "slab_ctas", "bulk", "fused", "BN", "KC", "npass", "TW", "TH", "coalesce", "tiles_x", "tiles_y", "tiles_n", "D",
+            "kchunks", "ntaps")
+    d = dict(zip(keys, list(info)))
+    d["instance"] = (d["slab_ctas"], d["bulk"], d["fused"], d["BN"], d["KC"])
+    return d
 
 
 def rel_err(a, b):
@@ -63,9 +77,18 @@ def rel_err(a, b):
 
 
 def tc_conv(x_cl, w, *, dil=1, npass=3, bias=None, scale=None, act_code=L.ACT_NONE, prelu=0.0, res_cl=None, res_after_act=0,
-            batch=None, stride=1, transposed=False, f16=0, q8_out=None):
+            batch=None, stride=1, transposed=False, f16=0, q8_out=None, geoms=None, cout=None, res_cstride=0, out_cstride=0,
+            out_coff=0, bias_per_batch=0, check_finite=0, out_f32=None, out_hi=None, out_lo=None, out_h16=None, out_q8=None,
+            num_sms=148, err=None, info_out=None, res_lo=None):
     """x_cl: fp32 [B,(D,)H,W,Cin] cpu; w: torch layout [Cout,Cin,(kd,)k,k] ([Cin,Cout,3,3,3] when transposed).
-    Returns (fp32 output, 16-bit output as fp32), cpu, channels-last."""
+    Returns (fp32 output, 16-bit output as fp32), cpu, channels-last.
+
+    The plan holds B = x_cl.shape[0] images; ``batch`` runs fewer.  ``geoms``: explicit tap tables (adp_tc_geom); w is then the
+    packed fp32 [w_taps, Cout(Pad), Cin] tensor and ``cout`` the real output channel count.  ``out_f32`` / ``out_hi`` /
+    ``out_lo`` / ``out_h16`` / ``out_q8``: device buffers the caller provides (pre-filled canaries stay where nothing is
+    written), or False for no such output; None = the default (fresh fp32 NaN / 16-bit zero planes, no h16 / q8 copy).
+    A returned value is None where there is no such output.  ``err``: the int32[2] device flag to pass (watchdog code must
+    stay 0).  ``info_out``: a list that receives plan_info() of every plan.  ``res_lo=False``: a bf16 residual without lo plane."""
     from rgbmanip_b200 import geometry
     from rgbmanip_b200.engine import pack_tc_weights
     lib = L.load()
@@ -73,9 +96,14 @@ def tc_conv(x_cl, w, *, dil=1, npass=3, bias=None, scale=None, act_code=L.ACT_NO
     B = x_cl.shape[0]
     D = x_cl.shape[1] if three_d else 1
     H, Wd, Cin = x_cl.shape[-3], x_cl.shape[-2], x_cl.shape[-1]
-    kd = w.shape[2] if three_d else 1
-    ks = w.shape[-1]
-    if transposed:
+    kd = w.shape[2] if (three_d and geoms is None) else 1
+    ks = w.shape[-1] if geoms is None else 1
+    if geoms is not None:
+        Cout = cout
+        wt = w.contiguous()
+        g0 = geoms[0]
+        oshape = (B, g0.oD, g0.oH, g0.oW, Cout) if three_d else (B, g0.oH, g0.oW, Cout)
+    elif transposed:
         Cout = w.shape[1]
         wt = w.reshape(Cin, Cout, -1).permute(2, 1, 0).contiguous()
         geoms = geometry.transposed_classes(D, H, Wd)
@@ -91,8 +119,8 @@ def tc_conv(x_cl, w, *, dil=1, npass=3, bias=None, scale=None, act_code=L.ACT_NO
             geoms = [None]
             oshape = tuple(x_cl.shape[:-1]) + (Cout,)
     cpad = (Cout + 15) // 16 * 16
-    if cpad != Cout:
-        wt = torch.cat([wt, torch.zeros(wt.shape[0], cpad - Cout, Cin)], 1).contiguous()
+    if wt.shape[1] < cpad:
+        wt = torch.cat([wt, torch.zeros(wt.shape[0], cpad - wt.shape[1], Cin)], 1).contiguous()
     wh, wl = (t.to(DEV).contiguous() if t is not None else None for t in pack_tc_weights(wt, f16, npass))
     xq = None
     if f16:
@@ -103,29 +131,41 @@ def tc_conv(x_cl, w, *, dil=1, npass=3, bias=None, scale=None, act_code=L.ACT_NO
     else:
         xh, xl = split(x_cl, npass == 3)
         dt16 = torch.bfloat16
-    out_f32 = torch.full(oshape, float("nan"), dtype=torch.float32, device=DEV)
-    out_hi = torch.zeros(out_f32.shape, dtype=dt16, device=DEV)
-    out_lo = torch.zeros_like(out_hi) if not f16 else None
+    if out_f32 is None:
+        out_f32 = torch.full(oshape, float("nan"), dtype=torch.float32, device=DEV)
+    if out_hi is None:
+        out_hi = torch.zeros(oshape, dtype=dt16, device=DEV)
+    if out_lo is None:
+        out_lo = torch.zeros(oshape, dtype=dt16, device=DEV) if not f16 else False
+    out_f32, out_hi, out_lo = (t if t is not False else None for t in (out_f32, out_hi, out_lo))
+    out_h16 = out_h16 if out_h16 is not False else None
     rh = rl = None
     if res_cl is not None:
         if f16:
             rh = res_cl.to(torch.float16).to(DEV).contiguous()
         else:
-            rh, rl = split(res_cl, True)
-    b_d = bias.to(DEV) if bias is not None else None
+            rh, rl = split(res_cl, res_lo is not False)
+    b_d = bias.to(DEV).contiguous() if bias is not None else None
     s_d = scale.to(DEV) if scale is not None else None
-    out_q8 = torch.zeros(out_f32.shape, dtype=torch.uint8, device=DEV) if q8_out is not None else None
-    ep = epilogue(out_hi, out_lo, out_f32, s_d, b_d, act_code, prelu, rh, rl, res_after_act, out_q8=out_q8)
+    if out_q8 is None or out_q8 is False:
+        out_q8 = torch.zeros(oshape, dtype=torch.uint8, device=DEV) if q8_out is not None else None
+    ep = epilogue(out_hi, out_lo, out_f32, s_d, b_d, act_code, prelu, rh, rl, res_after_act, out_q8=out_q8, res_cstride=res_cstride,
+                  out_h16=out_h16, out_cstride=out_cstride, out_coff=out_coff, bias_per_batch=bias_per_batch, check_finite=check_finite)
     a = act(xh, xl, B, D, H, Wd, Cin, f16, xq)
-    err = torch.zeros(2, dtype=torch.int32, device=DEV)
+    if err is None:
+        err = torch.zeros(2, dtype=torch.int32, device=DEV)
     for g in geoms:
         plan = C.c_void_p()
         L.check(lib.adp_conv_tc_plan(C.byref(plan), C.byref(a), L.ptr(wh), L.ptr(wl), Cout, kd, ks, dil, npass, C.byref(ep),
-                                     C.byref(g) if g is not None else None, 148), "plan")
-        L.check(lib.adp_conv_tc_run(plan, B if batch is None else batch, L.ptr(err), stream()), "run")
-        torch.cuda.synchronize()
-        lib.adp_conv_tc_free(plan)
+                                     C.byref(g) if g is not None else None, num_sms), "plan")
+        try:
+            if info_out is not None:
+                info_out.append(plan_info(plan))
+            L.check(lib.adp_conv_tc_run(plan, B if batch is None else batch, L.ptr(err), stream()), "run")
+            torch.cuda.synchronize()
+        finally:
+            lib.adp_conv_tc_free(plan)
     assert int(err[0].item()) == 0, f"watchdog code {int(err[0].item())}"
     if q8_out is not None:
         q8_out.append(from_e4m3(out_q8.cpu()) * 2.0)
-    return out_f32.cpu(), val(out_hi, out_lo).cpu()
+    return (out_f32.cpu() if out_f32 is not None else None), (val(out_hi, out_lo).cpu() if out_hi is not None else None)
