@@ -152,8 +152,9 @@ ADP_API int adp_pack_s2d(const float* crops, const adp_act* out, int batch, int 
  * out [B,D,H,W,16] (8 channels + 8 zero), folded BatchNorm + ReLU.  w: 16-bit [3 kx][4 chunks of 8 channels][80 n][8] with
  * n = (kz*3+ky)*8 + co (rows 72..79 zero): depth and row taps folded into the MMA's N (rgbmanip_b200.geometry.conv0_ring_weights).
  * flags: bit 0 must be 0 (reserved: planar volume layout); bit 1 (ADP_LAYOUT_S2D) = write the 8 real channels
- * space-to-depth(2): out [B,D/2,H/2,W/2,64], channel = ((d&1)*4 + (y&1)*2 + (x&1))*8 + co.  In that layout the stride-2
- * conv1 and the skip connection of the transposed conv11 (network_v5.py:265,278,283) read it as a stride-1 tensor. */
+ * space-to-depth(2): out [B,D/2,H/2,W/2,64] (D even, else ADP_ERR_ARG), channel = ((d&1)*4 + (y&1)*2 + (x&1))*8 + co.  In that
+ * layout the stride-2 conv1 and the skip connection of the transposed conv11 (network_v5.py:265,278,283) read it as a stride-1
+ * tensor. */
 #define ADP_LAYOUT_F16 1
 #define ADP_LAYOUT_S2D 2
 typedef struct adp_conv0_plan adp_conv0_plan;
@@ -189,7 +190,8 @@ ADP_API int adp_build_volume(const void* feat_ref, const void* feat_src, const f
  * (xfeat [B,P,32], xcat [B,P,96] columns 0..31); the per-point MLPs (network_v5.py:432-444,486-493) then run as 1x1
  * convolutions through adp_conv_tc_*; adp_colsum = sum over points (fixed-order, no atomics), adp_pose_gbias = per-env bias of
  * pose_mlp2's first layer, adp_rot_head = rotation MLP + Ortho6d2Mat (rotation_utils.py:18-27).
- * x11_format: ADP_LAYOUT_F16 (IEEE half instead of bf16) | ADP_LAYOUT_S2D (x11 stored [B,D/2,S/2,S/2,64], see adp_conv0_plan_create).
+ * x11_format: ADP_LAYOUT_F16 (IEEE half instead of bf16) | ADP_LAYOUT_S2D (x11 stored [B,D/2,S/2,S/2,64], S even, see
+ * adp_conv0_plan_create).
  * x11 == NULL selects the single-view mode (backbone + NOCS of one frame, network_v5.py:432-444): only xfeat is written. */
 ADP_API int adp_decode_gather(const float* feat_ref, const float* feat_src, const float* Mw, const float* depths, const void* x11,
                       const int32_t* choose, const uint8_t* valid, const float* prob_w, float* depth, void* xfeat_hi,

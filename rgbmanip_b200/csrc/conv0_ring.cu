@@ -281,6 +281,8 @@ int conv0_plan(Conv0Plan* pl, const Act& in, const uint16_t* w_packed, const flo
     ADP_TRY(tc_conv_init_driver());
     ADP_CHECK_ARG(in.C == 32 && in.W % C0_SEG == 0 && in.D >= 2 && in.H % C0_R == 0,
                   "conv0 ring kernel: C = 32, W % 112 == 0, D >= 2, H % 4 == 0");
+    // plane D-1 of an odd D would land at s2d depth (D-1)/2, one past the end of a [B, D/2, ...] output
+    ADP_CHECK_ARG(!(flags & 2) || in.D % 2 == 0, "conv0 ring kernel: the space-to-depth(2) output layout needs an even D");
     cuuint64_t dims[5] = {(cuuint64_t)in.C, (cuuint64_t)in.W, (cuuint64_t)in.H, (cuuint64_t)in.D, (cuuint64_t)in.B};
     cuuint64_t strides[4] = {(cuuint64_t)in.C * 2, (cuuint64_t)in.W * in.C * 2, (cuuint64_t)in.H * in.W * in.C * 2,
                              (cuuint64_t)in.D * in.H * in.W * in.C * 2};

@@ -327,6 +327,8 @@ rot_head_kernel(const float* __restrict__ psum, const uint8_t* __restrict__ vali
 int decode_gather_run(const DecodeArgs& a, const float* prob_w, bf16* xfeat_hi, bf16* xfeat_lo, bf16* xcat_hi, bf16* xcat_lo,
                       cudaStream_t stream) {
     ADP_CHECK_ARG(a.D == 24 && a.P % PB == 0, "24 depth hypotheses, P multiple of 32");
+    // row / column S-1 of an odd S would be read from s2d cell (S-1)/2, one past the end of a [B, D/2, S/2, S/2, 64] volume
+    ADP_CHECK_ARG(!a.x11 || !a.x11_s2d || a.S % 2 == 0, "decode gather: the space-to-depth(2) x11 layout needs an even S");
     if (a.B == 0) return ADP_OK;
     const size_t smem1 = (size_t)(2 * PB * LDS + PB * 24 + 216) * sizeof(float) + PB * sizeof(int);
     static_assert(PB * 9 * 24 <= PB * LDS, "the partial-logit scratch fits the first activation buffer");

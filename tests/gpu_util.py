@@ -76,6 +76,110 @@ def rel_err(a, b):
     return float((a - b).abs().max() / (b.abs().max() + 1e-30))
 
 
+# ------------------------------------------------------------------------------------------------ per-element comparison
+CANARY16, CANARY8 = 0x7E5A, 0x5A       # fill bits of output buffers: a 16-bit NaN / an fp8 byte no kernel computes here
+CANARY32 = 0x7FC00000                   # the fp32 quiet NaN torch writes for float("nan")
+
+
+def ulp(r, fmt):
+    """One unit in the last place of `fmt` at |r| (normal range; the smallest normal's ulp below it)."""
+    mant, emin = {"f16": (10, -14), "bf16": (7, -126)}[fmt]
+    _, e = torch.frexp(r.abs())
+    e = torch.where(r != 0, e - 1, torch.full_like(e, emin)).clamp_min(emin)
+    return torch.pow(2.0, (e - mant).double())
+
+
+def assert_close(got, ref, fmt, slack, what):
+    """Per element: |got - ref| <= slack (+ one ulp of a 16-bit format at |ref|, or 2^-16 |ref| for a bf16 hi + lo pair).
+    slack is a number or a tensor that broadcasts against ref.  Returns the largest error as a fraction of its bound."""
+    got = got.double()
+    err = (got - ref).abs()
+    bound = torch.zeros_like(ref) + slack
+    if fmt in ("f16", "bf16"):
+        bound = bound + ulp(ref, fmt)
+    elif fmt == "bf16x2":
+        bound = bound + ref.abs() * 2.0 ** -16
+    bad = ~(err <= bound)
+    if bad.any():
+        i = int(torch.nonzero(bad.reshape(-1))[0])
+        raise AssertionError(f"{what}: {int(bad.sum())} of {bad.numel()} elements out of bound; first at index "
+                             f"{tuple(np.unravel_index(i, tuple(ref.shape)))}: got {float(got.reshape(-1)[i])}, "
+                             f"ref {float(ref.reshape(-1)[i])}, bound {float(bound.reshape(-1)[i])}")
+    return float((err / bound).max())
+
+
+def bits(t):
+    """The raw bits of a tensor as an integer tensor of the same element size, on the CPU (NaN canaries compare equal)."""
+    return t.view({1: torch.uint8, 2: torch.int16, 4: torch.int32}[t.element_size()]).cpu()
+
+
+def canary16(shape, dt):
+    return torch.full(shape, CANARY16, dtype=torch.int16, device=DEV).view(dt)
+
+
+def canary32(shape):
+    return torch.full(shape, CANARY32, dtype=torch.int32, device=DEV).view(torch.float32)
+
+
+# ------------------------------------------------------------------------------------------------ thin runners of the
+# cost-regularisation kernels: the caller owns every buffer (so it can pre-fill canaries); batch < the plan's B runs part of it
+def _err_flag(err):
+    return torch.zeros(2, dtype=torch.int32, device=DEV) if err is None else err
+
+
+def conv0(vol, w_packed, scale, shift, out, *, flags=0, num_sms=148, batch=None, err=None):
+    """adp_conv0_plan_create + adp_conv0_run.  vol: device [B,D,H,W,32] fp16 or bf16 (its dtype sets the format); w_packed:
+    rgbmanip_b200.geometry.conv0_ring_weights in the same dtype; scale / shift: device fp32 [8]; out: [B,D,H,W,16] or, with
+    flags = LAYOUT_S2D, [B,D/2,H/2,W/2,64].  The plan holds B = vol.shape[0] images and runs `batch` of them."""
+    lib = L.load()
+    B, D, H, W, Cn = vol.shape
+    err = _err_flag(err)
+    a = act(vol, None, B, D, H, W, Cn, int(vol.dtype == torch.float16))
+    plan = C.c_void_p()
+    L.check(lib.adp_conv0_plan_create(C.byref(plan), C.byref(a), L.ptr(w_packed), L.ptr(scale), L.ptr(shift), L.ptr(out), flags,
+                                      num_sms), "conv0 plan")
+    try:
+        L.check(lib.adp_conv0_run(plan, B if batch is None else batch, L.ptr(err), stream()), "conv0 run")
+        torch.cuda.synchronize()
+    finally:
+        lib.adp_conv0_free(plan)
+    assert int(err[0].item()) == 0, f"watchdog code {int(err[0].item())}"
+    return out
+
+
+def tconv(x, w, cout, scale, bias, res, out, *, res_cstride=0, flags=0, num_sms=148, batch=None, err=None):
+    """adp_tconv_plan_create + adp_tconv_run.  x: device [B,D,H,W,Cin] fp16 or bf16; w: [27, pad16(cout), Cin] in the same
+    dtype; scale / bias: device fp32 [cout]; res: the skip tensor or None; out: [B,2D,2H,2W,cout] (or the s2d layout with
+    flags = LAYOUT_S2D).  The plan holds B = x.shape[0] images and runs `batch` of them."""
+    lib = L.load()
+    B, D, H, W, Cn = x.shape
+    err = _err_flag(err)
+    a = act(x, None, B, D, H, W, Cn, int(x.dtype == torch.float16))
+    plan = C.c_void_p()
+    L.check(lib.adp_tconv_plan_create(C.byref(plan), C.byref(a), L.ptr(w), cout, L.ptr(scale), L.ptr(bias), L.ptr(res), res_cstride,
+                                      L.ptr(out), flags, num_sms), "tconv plan")
+    try:
+        L.check(lib.adp_tconv_run(plan, B if batch is None else batch, L.ptr(err), stream()), "tconv run")
+        torch.cuda.synchronize()
+    finally:
+        lib.adp_tconv_free(plan)
+    assert int(err[0].item()) == 0, f"watchdog code {int(err[0].item())}"
+    return out
+
+
+def decode_gather(feat_ref, feat_src, Mw, depths, x11, choose, valid, prob_w, outs, *, batch, S, P, x11_format, D=24):
+    """adp_decode_gather over `batch` environments.  outs: dict of the caller's device buffers depth, xfeat_hi, xfeat_lo,
+    xcat_hi, xcat_lo, dbg_logits, dbg_fused (a missing key passes NULL).  x11 = None selects the single-view mode.  The kernel
+    has no pipeline and takes no error flag."""
+    lib = L.load()
+    o = {k: L.ptr(outs.get(k)) for k in ("depth", "xfeat_hi", "xfeat_lo", "xcat_hi", "xcat_lo", "dbg_logits", "dbg_fused")}
+    L.check(lib.adp_decode_gather(L.ptr(feat_ref), L.ptr(feat_src), L.ptr(Mw), L.ptr(depths), L.ptr(x11), L.ptr(choose), L.ptr(valid),
+                                  L.ptr(prob_w), o["depth"], o["xfeat_hi"], o["xfeat_lo"], o["xcat_hi"], o["xcat_lo"], o["dbg_logits"],
+                                  o["dbg_fused"], batch, S, D, P, x11_format, stream()), "decode_gather")
+    torch.cuda.synchronize()
+    return outs
+
+
 def tc_conv(x_cl, w, *, dil=1, npass=3, bias=None, scale=None, act_code=L.ACT_NONE, prelu=0.0, res_cl=None, res_after_act=0,
             batch=None, stride=1, transposed=False, f16=0, q8_out=None, geoms=None, cout=None, res_cstride=0, out_cstride=0,
             out_coff=0, bias_per_batch=0, check_finite=0, out_f32=None, out_hi=None, out_lo=None, out_h16=None, out_q8=None,

@@ -55,3 +55,17 @@ def test_stem_s2d_weights_match_7x7_stride2():
             s2d[0, 0, :, :, (py * 2 + px) * 3:(py * 2 + px) * 3 + 3] = cl[0, py::2, px::2]
     got = _run_taps(s2d, G.stem_s2d_weights(w).double(), G.stem_s2d(16))
     assert float((got[0, 0].permute(2, 0, 1) - ref[0]).abs().max()) < 1e-5
+
+
+def test_conv0_ring_weights_layout():
+    """adp_conv0_run reads w[co, c, kz, ky, kx] at [kx][c // 8][(kz * 3 + ky) * 8 + co][c % 8]; rows 72..79 of N are zero."""
+    w = torch.randn(8, 32, 3, 3, 3)
+    p = G.conv0_ring_weights(w)
+    assert p.shape == (3, 4, 80, 8)
+    for co in range(8):
+        for c in range(32):
+            for kz in range(3):
+                for ky in range(3):
+                    for kx in range(3):
+                        assert p[kx, c // 8, (kz * 3 + ky) * 8 + co, c % 8] == w[co, c, kz, ky, kx]
+    assert (p[:, :, 72:] == 0).all()

@@ -26,6 +26,7 @@ import numpy as np
 import pytest
 import torch
 
+from gpu_util import CANARY8, CANARY16, assert_close, bits, canary16
 from rgbmanip_b200 import _lib as L
 from rgbmanip_b200 import geometry, weights
 
@@ -51,7 +52,6 @@ def inst_name(inst):
 
 SPLIT_TOL = {2: 2e-5, 3: 2e-4, 4: 3e-5}       # npass -> bound relative to max|ref| (test_gpu_stages.py derives them)
 ONE_PASS_TOL = 1e-5                           # fp32 accumulation order with exact operands
-CANARY16, CANARY8 = 0x7E5A, 0x5A
 
 
 @dataclass
@@ -311,37 +311,7 @@ def reference(case, d, w_exact=None):
     return v
 
 
-def ulp(r, fmt):
-    """One unit in the last place of `fmt` at |r| (normal range; the smallest normal's ulp below it)."""
-    mant, emin = {"f16": (10, -14), "bf16": (7, -126)}[fmt]
-    _, e = torch.frexp(r.abs())
-    e = torch.where(r != 0, e - 1, torch.full_like(e, emin)).clamp_min(emin)
-    return torch.pow(2.0, (e - mant).double())
-
-
-def assert_close(got, ref, fmt, slack, what):
-    """Per element: |got - ref| <= slack (+ one ulp of a 16-bit format at |ref|, or 2^-16 |ref| for a bf16 hi + lo pair).
-    Returns the largest error as a fraction of its bound."""
-    got = got.double()
-    err = (got - ref).abs()
-    bound = torch.full_like(ref, slack)
-    if fmt in ("f16", "bf16"):
-        bound = bound + ulp(ref, fmt)
-    elif fmt == "bf16x2":
-        bound = bound + ref.abs() * 2.0 ** -16
-    bad = ~(err <= bound)
-    if bad.any():
-        i = int(torch.nonzero(bad.reshape(-1))[0])
-        raise AssertionError(f"{what}: {int(bad.sum())} of {bad.numel()} elements out of bound; first at flat index {i}: "
-                             f"got {float(got.reshape(-1)[i])}, ref {float(ref.reshape(-1)[i])}, bound {float(bound.reshape(-1)[i])}")
-    return float((err / bound).max())
-
-
 # ------------------------------------------------------------------------------------------------ running a case
-def _canary16(shape, dt):
-    return torch.full(shape, CANARY16, dtype=torch.int16, device="cuda:0").view(dt)
-
-
 def run(G, case, d, *, num_sms=148, batch=None, rng=None, x=None, err=None):
     """One adp_conv_tc run of the case into freshly canary-filled output buffers.  rng = (out_cstride, out_coff) overrides the
     layer's channel range ((0, 0) = dense).  Returns (buffers, plan infos, err flag)."""
@@ -350,9 +320,9 @@ def run(G, case, d, *, num_sms=148, batch=None, rng=None, x=None, err=None):
     dt16 = torch.float16 if case.f16 else torch.bfloat16
     outs = case.outs.split()
     bufs = dict(out_f32=torch.full(d.oshape, float("nan"), device="cuda:0") if "f32" in outs else False,
-                out_hi=_canary16(wide, dt16) if "hi" in outs else False,
-                out_lo=_canary16(wide, dt16) if "lo" in outs else False,
-                out_h16=_canary16(d.oshape, torch.float16) if "h16" in outs else False,
+                out_hi=canary16(wide, dt16) if "hi" in outs else False,
+                out_lo=canary16(wide, dt16) if "lo" in outs else False,
+                out_h16=canary16(d.oshape, torch.float16) if "h16" in outs else False,
                 out_q8=torch.full(wide, CANARY8, dtype=torch.uint8, device="cuda:0") if "q8" in outs else False)
     info = []
     if err is None:
@@ -376,10 +346,6 @@ def full_run(G, case):
     if case.id not in _FULL:
         _FULL[case.id] = run(G, case, built(case))
     return _FULL[case.id]
-
-
-def bits(t):
-    return t.view({1: torch.uint8, 2: torch.int16, 4: torch.int32}[t.element_size()]).cpu()
 
 
 # ------------------------------------------------------------------------------------------------ (a) instance coverage
@@ -609,7 +575,7 @@ def test_fp8_twin_needs_coalesced_aligned_range(G):
         with pytest.raises(L.AdpError, match=r"out_q8 .*" + why):
             G.tc_conv(x, w, npass=2, f16=1, act_code=L.ACT_RELU, out_f32=False, out_hi=hi, out_q8=q8, out_cstride=cs, out_coff=coff)
     coff = 16
-    hi = _canary16((B, H, W, cs), torch.float16)
+    hi = canary16((B, H, W, cs), torch.float16)
     q8 = torch.full((B, H, W, cs), CANARY8, dtype=torch.uint8, device=G.DEV)
     f32 = torch.full((B, H, W, Cout), float("nan"), device=G.DEV)
     G.tc_conv(x, w, npass=2, f16=1, act_code=L.ACT_RELU, out_f32=f32, out_hi=hi, out_q8=q8, out_cstride=cs, out_coff=coff)
