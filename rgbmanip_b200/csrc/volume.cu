@@ -18,7 +18,7 @@ namespace adp {
 // The kernel was bound by instruction issue (529 warp instructions per voxel and plane, now 286), so the inner loop is kept
 // lean: the bilinear blend runs on the mixed-precision
 // FMA (fhfma8: the fp16 feature times the fp16-rounded bilinear weight, exact product, fp32 accumulation - the weight rounding
-// of <= 2^-12 relative per corner sits below the fp16 storage rounding of the result), the per-voxel projection uses one
+// of <= 2^-11 relative per corner sits below the fp16 storage rounding of the result), the per-voxel projection uses one
 // reciprocal instead of four divisions (sample positions agree with the reference's expression to ~5e-5 px), and the footprint
 // is staged row by row (no integer divisions).
 constexpr int VT_T = 16;
@@ -163,6 +163,12 @@ build_volume_tile_kernel(const __half* __restrict__ f_ref, const __half* __restr
         const int bx0 = some ? max(box[0], 0) : 0, by0 = some ? max(box[1], 0) : 0;
         const int bx1 = some ? min(box[2], W - 1) : -1, by1 = some ? min(box[3], H - 1) : -1;
         const int bw = bx1 - bx0 + 1, bh = by1 - by0 + 1;
+        // Reset the other parity's box for plane d + 1 here, between A and B.  Its last readers (plane d - 1, between its own A
+        // and B) are done before this plane's A, and its next writers (plane d + 1's atomics) start after this plane's B.  After B
+        // the reset would be unordered against a faster warp's plane-(d + 1) atomics and could erase its extents.  A plane that
+        // takes the empty shortcut above skips this reset, so the plane after it starts from the box of the plane two before:
+        // a superset of its own box, which can only turn a staged plane into a fallback one, never drop a pixel.
+        if (tid < 4) s_box[(d + 1) & 1][tid] = (tid & 2) ? INT_MIN : INT_MAX;
         const bool staged = bw > 0 && bh > 0 && bw * bh <= VT_MAXPX;       // uniform over the block
         if (staged) {           // a warp per footprint row (bw x 64 contiguous bytes, lane -> (pixel, 16-byte chunk)), every copy in flight at once;
                                 // through L1: neighbouring planes and tiles re-read most of the footprint (.ca 1.51 ms, .cg 1.65 ms per chunk)
@@ -175,8 +181,6 @@ build_volume_tile_kernel(const __half* __restrict__ f_ref, const __half* __restr
             cp_async_wait_all();
         }
         __syncthreads();                         // B: the footprint is staged
-        // the other parity's box was last read before B of the previous plane: reset it for the next plane
-        if (tid < 4) s_box[(d + 1) & 1][tid] = (tid & 2) ? INT_MIN : INT_MAX;
         uint32_t wk[4];         // the weights as fp16 multipliers of the mixed-precision FMA (0 where a corner is outside)
         wk[0] = __half_as_ushort(__float2half_rn(bl.w00)); wk[1] = __half_as_ushort(__float2half_rn(bl.w01));
         wk[2] = __half_as_ushort(__float2half_rn(bl.w10)); wk[3] = __half_as_ushort(__float2half_rn(bl.w11));

@@ -180,6 +180,19 @@ def decode_gather(feat_ref, feat_src, Mw, depths, x11, choose, valid, prob_w, ou
     return outs
 
 
+def volume(feat_ref, feat_src, Mw, depths, out, *, batch=None):
+    """adp_build_volume over `batch` environments (default out.shape[0]).  feat_ref / feat_src: device fp16 [>= batch, H, W, 32];
+    Mw: device fp32 [>= batch, 12]; depths: device fp32 [D]; out: the caller's [>= batch, D, H, W, 32] buffer, fp16 or bf16
+    (its dtype selects the output format)."""
+    _, D, H, W, Cn = out.shape
+    assert depths.numel() == D and out.dtype in (torch.float16, torch.bfloat16)
+    L.check(L.load().adp_build_volume(L.ptr(feat_ref), L.ptr(feat_src), L.ptr(Mw), L.ptr(depths), L.ptr(out),
+                                      out.shape[0] if batch is None else batch, D, H, W, Cn, int(out.dtype == torch.float16),
+                                      stream()), "build_volume")
+    torch.cuda.synchronize()
+    return out
+
+
 def tc_conv(x_cl, w, *, dil=1, npass=3, bias=None, scale=None, act_code=L.ACT_NONE, prelu=0.0, res_cl=None, res_after_act=0,
             batch=None, stride=1, transposed=False, f16=0, q8_out=None, geoms=None, cout=None, res_cstride=0, out_cstride=0,
             out_coff=0, bias_per_batch=0, check_finite=0, out_f32=None, out_hi=None, out_lo=None, out_h16=None, out_q8=None,

@@ -317,10 +317,10 @@ def decode_data(G):
         np.random.seed(3)
         kp1 = np.stack([O.prepare_model_input(batch.rgb1[e], batch.mask1[e], batch.K[e])[3] for e in range(B)])
         kp2 = np.stack([O.prepare_model_input(batch.rgb2[e], batch.mask2[e], batch.K[e])[3] for e in range(B)])
-        dev = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(G.DEV)
+        # the camera buffers stay referenced until the kernel has run (L.ptr holds no reference; freed temporaries would alias)
+        cams = [torch.from_numpy(np.ascontiguousarray(a).reshape(B, -1)).to(G.DEV) for a in (kp1, batch.E1, kp2, batch.E2)]
         Mw = torch.zeros((B, 12), device=G.DEV)
-        L.check(L.load().adp_warp_matrices(L.ptr(dev(kp1.reshape(B, 9))), L.ptr(dev(batch.E1.reshape(B, 16))), L.ptr(dev(kp2.reshape(B, 9))),
-                                           L.ptr(dev(batch.E2.reshape(B, 16))), L.ptr(Mw), None, None, None, B, G.stream()), "warp matrices")
+        L.check(L.load().adp_warp_matrices(*(L.ptr(t) for t in cams), L.ptr(Mw), None, None, None, B, G.stream()), "warp matrices")
         torch.cuda.synchronize()
         d = SimpleNamespace(feat_ref=_t(rng, B, S, S, 32), feat_src=_t(rng, B, S, S, 32), Mw=Mw.cpu(),
                             depths=torch.from_numpy(O.depth_hypotheses()), x11=_t(rng, B, DEC_D, S, S, 8),
