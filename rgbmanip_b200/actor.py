@@ -27,6 +27,13 @@ class DeviceActor:
         self.activation = ACTIVATIONS[activation]
         self.lib = L.load()
         self.ring = ring
+        self.shards = None
+        if hasattr(ring, "shards"):
+            # a ring sharded over devices: the weights are replicated on every shard's device and each shard's actor reads its
+            # own queues (an observation depends on its environment's queues and the step only)
+            self.shards = [DeviceActor(actor_state_dict, s, activation) for s in ring.shards]
+            self.dims = self.shards[0].dims
+            return
         dev = ring.device
         sd = {k.replace("actor_critic.", ""): v for k, v in actor_state_dict.items()}
         idx = sorted({int(k.split(".")[1]) for k in sd if k.startswith("actor.") and k.endswith(".weight")})
@@ -51,6 +58,12 @@ class DeviceActor:
         step = (r.accumulate_steps if accumulate_steps is None else accumulate_steps) - 1
         if not 0 <= step < r.max_steps:
             raise IndexError(f"one_hot index {step} outside [0, {r.max_steps})")       # torch.nn.functional.one_hot raises too
+        if self.shards is not None:          # -> [N, A] / [N, T*12] in env order on the first device
+            outs = []
+            for a in self.shards:
+                with torch.cuda.device(a.ring.device):
+                    outs.append(a.act_inference(step + 1))
+            return tuple(torch.cat([o[i].to(r.device) for o in outs]) for i in (0, 1))
         st = C.c_void_p(torch.cuda.current_stream(r.device).cuda_stream)
         L.check(self.lib.adp_actor_forward(L.ptr(r.pose), L.ptr(r.bbox), r.max_steps, r.num_envs, step, len(self.W), self._dims,
                                            self._wp, self._bp, self.activation, L.ptr(self.obs), L.ptr(self.act), st), "actor_forward")

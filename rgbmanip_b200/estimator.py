@@ -201,7 +201,13 @@ class AdaPoseEstimator_v5(BasePoseEstimator):
         self._first_chunk = int(cfg.get("first_chunk_envs", 16))
 
     def _ensure_capacity(self, N):
-        """Auto-sized workspace: rebuild the engine with a larger chunk capacity the first time a bigger batch shows up."""
+        """Auto-sized workspace: rebuild the engine with a larger chunk capacity the first time a bigger batch shows up.  A
+        multi-device estimator grows every replica to its share of N (the contiguous block :meth:`_estimate_multi` gives it)."""
+        if self._replicas is not None:
+            from .dist import shard_range
+            world = len(self._replicas)
+            self._on_replicas(lambda r: self._replicas[r]._ensure_capacity(len(range(*shard_range(int(N), r, world)[:2]))))
+            return
         eng = self.estimator
         want = min(max(int(N), 1), AUTO_CHUNK_MAX)
         if not self._auto_chunk or want <= eng.E:
@@ -213,6 +219,26 @@ class AdaPoseEstimator_v5(BasePoseEstimator):
         self._stage_bufs, self._win_state, self._slot_free = {}, {}, [None, None]
         torch.cuda.empty_cache()
         self.estimator = Engine(sd, max_envs=want, **self._engine_args)
+
+    def one_device_chunk(self, N):
+        """Chunk capacity (environments) a one-device estimator of this configuration has for a batch of N environments: the
+        explicit ``max_envs`` / ``max_envs_per_chunk``, else the auto-sized 16 .. AUTO_CHUNK_MAX.  The view ring keys its random
+        draws by these chunks, so that a ring sharded over several devices draws what a one-device ring draws."""
+        rep = self._replicas[0] if self._replicas is not None else self
+        if not rep._auto_chunk:
+            return rep.estimator.E
+        return max(16, min(int(N), AUTO_CHUNK_MAX))
+
+    def _on_replicas(self, fn, which=None):
+        """``fn(r)`` for every replica index r (or those in ``which``), concurrently on the per-device host threads -> results in
+        order.  Pool threads are not tied to a replica: a thread re-pins itself to the GPU's NUMA node when its replica changes."""
+        def run(r):
+            if getattr(self._tls, "bound", None) != r:
+                from .dist import bind_to_gpu_numa
+                bind_to_gpu_numa(self._replicas[r].device)
+                self._tls.bound = r
+            return fn(r)
+        return list(self._pool.map(run, range(len(self._replicas)) if which is None else which))
 
     # -- helpers ---------------------------------------------------------------------------------
     _RGB_OK = (torch.uint8, torch.float32, torch.float64)
@@ -417,10 +443,14 @@ class AdaPoseEstimator_v5(BasePoseEstimator):
                            K.cpu().numpy().reshape(-1, 3, 3), E1.cpu().numpy().reshape(-1, 4, 4))
         return torch.from_numpy(box).to(self.device)
 
-    def estimate_nocs_single_view(self, camera_intrinsic_batch, rgb_batch, mask_batch, choose=None):
+    def estimate_nocs_single_view(self, camera_intrinsic_batch, rgb_batch, mask_batch, choose=None, env_offset=0, sample_seed=None):
         """BASELINE configs[0..1]: one view per environment -> (nocs [N,1024,3] float32, choose [N,1024] int32, valid [N] bool)
         as numpy arrays.  This is the per-view part of the reference forward (preprocessing, PSPNet, ``instance_color`` +
-        ``nocs_head``, network_v5.py:432-444); a full pose needs two views (interface_v5.py:256-257)."""
+        ``nocs_head``, network_v5.py:432-444); a full pose needs two views (interface_v5.py:256-257).  ``env_offset`` /
+        ``sample_seed`` as in :meth:`estimate`: a multi-device estimator runs one contiguous block per replica with the global
+        env index as the sampler key, so the result equals the one-device result bit for bit."""
+        if self._replicas is not None:
+            return self._single_view_multi(camera_intrinsic_batch, rgb_batch, mask_batch, choose, env_offset, sample_seed)
         self._ensure_capacity(len(camera_intrinsic_batch))
         eng = self.estimator
         K_b, rgb_b, m_b = (self._as_tensor(a) for a in (camera_intrinsic_batch, rgb_batch, mask_batch))
@@ -429,6 +459,7 @@ class AdaPoseEstimator_v5(BasePoseEstimator):
         chs = torch.empty((N, eng.P), dtype=torch.int32, device=self.device)
         val = torch.empty((N,), dtype=torch.uint8, device=self.device)
         self._calls += 1
+        seed = (self._seed + 7919 * self._calls) if sample_seed is None else int(sample_seed)
         with torch.cuda.device(self.device):
             for lo, hi in chunk_bounds(N, eng.E):
                 m = m_b[lo:hi]
@@ -439,7 +470,7 @@ class AdaPoseEstimator_v5(BasePoseEstimator):
                 c = None if choose is None else self._as_tensor(choose[lo:hi]).to(torch.int32).to(self.device)
                 n_, c_, v_ = eng.single_view_nocs(self._upload("rgb1", 0, rgb_b[lo:hi], self._rgb_dtype(rgb_b)),
                                                   self._upload("m1", 0, m), self._upload("K", 0, K_b[lo:hi], torch.float64), hi - lo,
-                                                  seed=self._seed + 7919 * self._calls, choose=c, env0=lo)
+                                                  seed=seed, choose=c, env0=int(env_offset) + lo)
                 nocs[lo:hi].copy_(n_); chs[lo:hi].copy_(c_); val[lo:hi].copy_(v_)
                 torch.cuda.current_stream(self.device).synchronize()       # the pinned staging slot is reused by the next chunk
             out = (nocs.cpu().numpy(), chs.cpu().numpy(), val.cpu().numpy().astype(bool))
@@ -460,16 +491,11 @@ class AdaPoseEstimator_v5(BasePoseEstimator):
             lo, hi, _ = shard_range(N, r, world)
             if hi <= lo:
                 return None
-            rep = self._replicas[r]
-            if getattr(self._tls, "bound", None) != r:      # pool threads are not tied to a replica: re-pin when it changes
-                from .dist import bind_to_gpu_numa
-                bind_to_gpu_numa(rep.device)
-                self._tls.bound = r
             sl = lambda a: None if a is None else a[lo:hi]
             ch = None if choose is None else (choose[0][lo:hi], choose[1][lo:hi])
-            return rep.estimate(*[a[lo:hi] for a in batches], choose=ch, return_tensor=True, ransac_idx=sl(ransac_idx),
-                                env_offset=int(env_offset) + lo, sample_seed=seed)
-        parts = [p for p in self._pool.map(run, range(world)) if p is not None]
+            return self._replicas[r].estimate(*[a[lo:hi] for a in batches], choose=ch, return_tensor=True, ransac_idx=sl(ransac_idx),
+                                              env_offset=int(env_offset) + lo, sample_seed=seed)
+        parts = [p for p in self._on_replicas(run) if p is not None]
         if return_tensor:
             if not parts:
                 return torch.empty((0, 8, 3), dtype=torch.float64, device=self.device)
@@ -477,6 +503,27 @@ class AdaPoseEstimator_v5(BasePoseEstimator):
         res = np.concatenate([p.cpu().numpy() for p in parts]) if parts else np.zeros((0, 8, 3))
         self.check_error_flag()
         return res
+
+    def _single_view_multi(self, K_b, rgb_b, m_b, choose, env_offset, sample_seed):
+        """:meth:`estimate_nocs_single_view` over the replicas: the blocks of :meth:`_estimate_multi`, gathered in env order."""
+        from .dist import shard_range
+        N = len(K_b)
+        world = len(self._replicas)
+        self._calls += 1
+        seed = (self._seed + 7919 * self._calls) if sample_seed is None else int(sample_seed)
+
+        def run(r):
+            lo, hi, _ = shard_range(N, r, world)
+            if hi <= lo:
+                return None
+            return self._replicas[r].estimate_nocs_single_view(K_b[lo:hi], rgb_b[lo:hi], m_b[lo:hi],
+                                                               choose=None if choose is None else choose[lo:hi],
+                                                               env_offset=int(env_offset) + lo, sample_seed=seed)
+        parts = [p for p in self._on_replicas(run) if p is not None]
+        if not parts:
+            rep = self._replicas[0].estimator
+            return np.zeros((0, rep.P, 3), np.float32), np.zeros((0, rep.P), np.int32), np.zeros((0,), bool)
+        return tuple(np.concatenate([p[i] for p in parts]) for i in range(3))
 
     def check_error_flag(self):
         """Synchronise and raise if the pipeline watchdog or the fp16 range guard fired (the tensor-returning paths defer it)."""
