@@ -4,27 +4,13 @@
 // One kernel: a block carries ACT_ENVS environments, the observation is assembled straight from the device-resident
 // queues (float64 -> float32 like the reference's .float()), activations ping-pong in shared memory, weights are read
 // through the read-only path (74 KB for the shipped sizes: L1/L2 resident).  fp32 throughout.
-#include "common.cuh"
+#include "stages.cuh"
 
 namespace adp {
 
 constexpr int ACT_ENVS = 8;
 constexpr int ACT_THREADS = 256;
 constexpr int ACT_MAXW = 256;       // widest layer
-constexpr int ACT_MAXL = 8;
-
-struct ActorArgs {
-    const double* pose;      // [T, N, 7]
-    const double* bbox;      // [T, N, 4]
-    int T, N, step;          // step = accumulate_steps - 1 (one-hot index)
-    int nlayers;
-    int activation;          // hidden activation, get_activation() of module.py:110-126: 0 elu, 1 selu, 2 relu/crelu, 3 lrelu, 4 tanh, 5 sigmoid
-    int dims[ACT_MAXL + 1];  // dims[0] = T * 12
-    const float* W[ACT_MAXL];   // torch layout [out][in]
-    const float* b[ACT_MAXL];
-    float* obs_out;          // [N, dims[0]] or nullptr
-    float* act_out;          // [N, dims[nlayers]]
-};
 
 __global__ void __launch_bounds__(ACT_THREADS)
 actor_forward_kernel(const ActorArgs a) {

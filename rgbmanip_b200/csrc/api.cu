@@ -4,8 +4,7 @@
 #include <atomic>
 #include <mutex>
 
-#include "../../include/adapose_b200.h"
-#include "common.cuh"
+#include "stages.cuh"
 #include "tc_conv.cuh"
 
 namespace adp {
@@ -19,63 +18,6 @@ void set_last_error(const char* fmt, ...) {
     vsnprintf(g_err, sizeof(g_err), fmt, ap);
     va_end(ap);
 }
-
-// implemented in the stage translation units
-int maxpool3x3s2(const Act& in, const Act& out, int batch, cudaStream_t stream);
-int psp_priors(const Act& feat, int feat_cs, const float* w, float* pooled, float* priors, int batch, cudaStream_t stream);
-int psp_fill_priors(const float* priors, const Act& out, int coff, int batch, cudaStream_t stream);
-int upsample2x(const Act& in, const Act& out, int batch, cudaStream_t stream);
-int upconv_blend(const Act& q, const Act& out, const float* bias, float slope, int batch, cudaStream_t stream);
-int pack_s2d(const float* crops, const Act& out, int batch, int S, cudaStream_t stream);
-int preprocess_run(const void* rgb, int rgb_dt, const void* mask, int mask_dt, const double* K, int k_stride, int F, int H, int W,
-                   int S, int P, uint32_t seed, int choose_mode, int frame_id0, int* bbox_ws, int* win, double* Kp, uint8_t* valid,
-                   float* crops, int* choose, int* counts, cudaStream_t stream);
-int mask_windows_run(const void* mask, int mask_dt, int F, int H, int W, int* bbox_ws, int* win, uint8_t* valid, cudaStream_t stream);
-int build_volume(const void* f_ref, const void* f_src, const float* Mw, const float* depths, bf16* vol, int B, int D, int H,
-                 int W, int C, int f16, cudaStream_t stream);
-int warp_matrices(const double* Kp_ref, const double* E_ref, const double* Kp_src, const double* E_src, float* Mw,
-                  const uint8_t* valid_ref, const uint8_t* valid_src, uint8_t* valid_env, int B, cudaStream_t stream);
-int fit_run(const float* nocs, const float* depth, const int* choose, const double* Kp, const float* R, const double* E,
-            const uint8_t* valid, double* bbox, double* scale_out, double* trans_out, const float* pts_cam, const int* pts_count,
-            int B, int P, int S, cudaStream_t stream);
-int nocs_match_run(const float* nocs1, const float* nocs2, const int* choose1, const int* choose2, const int* win1, const int* win2,
-                   const double* K, const double* E1, const double* E2, const uint8_t* valid, int S, float* pts2d1, float* pts_cam,
-                   float* nocs_m, int* count, int* match_ids, int B, int P, cudaStream_t stream);
-int view_fusion_run(const float* feat1, const float* feat2, const int* choose1, const int* choose2, const uint8_t* valid,
-                    const float* blocks, const float* depth_w, float* scratch, float* depth1, float* depth2, bf16* xcat_hi,
-                    bf16* xcat_lo, float* fused1, float* fused2, int B, int S, int P, int n_blocks, cudaStream_t stream);
-
-int fit_umeyama_run(const float* nocs, const float* depth, const int* choose, const double* Kp, const double* E, const uint8_t* valid,
-                    const int* rand_idx, uint32_t seed, double* bbox, double* scale_out, double* rot_out, double* trans_out, int B,
-                    int P, int S, cudaStream_t stream);
-struct Conv0Plan;
-Conv0Plan* conv0_alloc();
-void conv0_release(Conv0Plan* p);
-int conv0_plan(Conv0Plan* pl, const Act& in, const uint16_t* w_packed, const float* scale, const float* shift, uint16_t* out,
-               int planar, int num_sms);
-int conv0_run(Conv0Plan* pl, int batch, int* err_flag, cudaStream_t stream);
-
-int decode_gather_c(const float* feat_ref, const float* feat_src, const float* Mw, const float* depths, const void* x11,
-                    const int* choose, const uint8_t* valid, const float* prob_w, float* depth, void* xfeat_hi, void* xfeat_lo,
-                    void* xcat_hi, void* xcat_lo, float* dbg_logits, float* dbg_fused, int B, int S, int D, int P, int x11_f16,
-                    cudaStream_t stream);
-int colsum_run(const bf16* hi, const bf16* lo, const uint8_t* valid, float* out, int B, int P, int C, cudaStream_t stream);
-int pose_gbias_run(const float* gsum, const float* q0_w, const float* q0_b, const uint8_t* valid, float* gb, int B, int P,
-                   cudaStream_t stream);
-int rot_head_run(const float* psum, const uint8_t* valid, float* Rout, float* r6out, const adp_decode_weights* cw, int B, int P,
-                 cudaStream_t stream);
-constexpr int ACT_MAXL_API = 8;
-struct ActorArgs {
-    const double* pose; const double* bbox; int T, N, step; int nlayers; int activation; int dims[ACT_MAXL_API + 1];
-    const float* W[ACT_MAXL_API]; const float* b[ACT_MAXL_API]; float* obs_out; float* act_out;
-};
-int actor_forward(const ActorArgs& a, cudaStream_t stream);
-struct TconvPlan;
-TconvPlan* tconv_alloc();
-void tconv_release(TconvPlan* p);
-int tconv_plan(TconvPlan* pl, const Act& in, const bf16* w, int Cout, const float* scale, const float* bias, const bf16* res,
-               int res_cs, bf16* out, int flags, int num_sms);
-int tconv_run(TconvPlan* pl, int batch, int* err_flag, cudaStream_t stream);
 
 static Act to_act(const adp_act* a) {
     Act r;
@@ -131,15 +73,8 @@ int adp_conv_tc_plan(adp_conv_plan** plan, const adp_act* in, const void* w_hi, 
     ADP_CHECK_ARG(plan && in && w_hi && ep, "null pointer");
     ADP_CHECK_ARG(ep->out_hi || ep->out_f32, "epilogue has no output");
     adp_conv_plan* pl = new adp_conv_plan();
-    TcGeom g;
-    if (geom) {
-        g.ntaps = geom->ntaps;
-        for (int t = 0; t < 32; ++t) { g.dz[t] = geom->dz[t]; g.dy[t] = geom->dy[t]; g.dx[t] = geom->dx[t]; g.wt[t] = geom->wt[t]; }
-        g.in_mul = geom->in_mul; g.out_mul = geom->out_mul; g.out_oz = geom->out_oz; g.out_oy = geom->out_oy; g.out_ox = geom->out_ox;
-        g.gD = geom->gD; g.gH = geom->gH; g.gW = geom->gW; g.oD = geom->oD; g.oH = geom->oH; g.oW = geom->oW; g.w_taps = geom->w_taps;
-    }
     int r = tc_conv_plan(&pl->layer, to_act(in), reinterpret_cast<const bf16*>(w_hi), reinterpret_cast<const bf16*>(w_lo), cout,
-                         kd, ks, dil, npass, geom ? &g : nullptr, in->f16);
+                         kd, ks, dil, npass, geom, in->f16);
     if (r != ADP_OK) {
         delete pl;
         return r;
@@ -225,11 +160,11 @@ int adp_upconv_blend(const adp_act* q, const adp_act* out, const float* bias, fl
 }
 
 int adp_conv0_plan_create(adp_conv0_plan** plan, const adp_act* vol, const void* w_packed, const float* scale, const float* shift,
-                          void* out, int vol_planar, int num_sms) {
+                          void* out, int flags, int num_sms) {
     ADP_CHECK_ARG(plan && vol && w_packed && scale && shift && out, "null pointer");
     Conv0Plan* pl = conv0_alloc();
     int r = conv0_plan(pl, to_act(vol), reinterpret_cast<const uint16_t*>(w_packed), scale, shift, reinterpret_cast<uint16_t*>(out),
-                       vol_planar, num_sms);
+                       flags, num_sms);
     if (r != ADP_OK) {
         conv0_release(pl);
         return r;
@@ -321,7 +256,7 @@ int adp_actor_forward(const double* pose_queue, const double* bbox_queue, int T,
                       const float* const* weights, const float* const* biases, int activation, float* obs_out, float* act_out,
                       void* stream) {
     ADP_CHECK_ARG(pose_queue && bbox_queue && dims && weights && biases && act_out, "null pointer");
-    ADP_CHECK_ARG(nlayers >= 1 && nlayers <= ACT_MAXL_API, "1..8 layers");
+    ADP_CHECK_ARG(nlayers >= 1 && nlayers <= ACT_MAXL, "1..8 layers");
     ActorArgs a{};
     a.pose = pose_queue; a.bbox = bbox_queue; a.T = T; a.N = N; a.step = step; a.nlayers = nlayers; a.activation = activation;
     for (int l = 0; l <= nlayers; ++l) a.dims[l] = dims[l];

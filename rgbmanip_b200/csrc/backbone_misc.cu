@@ -1,7 +1,7 @@
 // Memory-bound helpers of the PSPNet backbone (channels-last, hi(+lo) bf16 activations):
 // 3x3/2 max-pool, pyramid pooling + 1x1 convs, pyramid concat fused with the first x2 bilinear upsample,
 // plain x2 bilinear upsample (align_corners=True).  Reference: ADA/lib/pspnet.py:66-107,142-158.
-#include "common.cuh"
+#include "stages.cuh"
 
 namespace adp {
 

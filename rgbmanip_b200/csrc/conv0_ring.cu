@@ -17,11 +17,9 @@
 // lands in one slot of a six-deep 80-column TMEM ring; the epilogue warps pull a slot out once, release it at once, and add its
 // nine 8-column groups into three register accumulators per output row (output planes d'-1, d', d'+1), apply the folded
 // BatchNorm + ReLU when a plane is complete and store 16 channels (8 real + 8 zero: conv1 needs Cin = 16 for the K = 16 MMA).
-#include "common.cuh"
 #include "ptx.cuh"
-
-#include <cudaTypedefs.h>
-#include <stdlib.h>
+#include "stages.cuh"
+#include "tma.cuh"
 
 namespace adp {
 
@@ -48,22 +46,6 @@ struct Conv0Params {
     int out_s2d;
     int* err;
 };
-
-// A operand: K-major, 64-byte swizzle (rows of 64 B = 32 channels; one MMA consumes 32 B of each row), SBO = 8 rows.
-__device__ __forceinline__ uint64_t make_desc_sw64(uint32_t addr) {
-    return (uint64_t)((addr & 0x3FFFF) >> 4) | (1ull << 16) | ((uint64_t)(512 >> 4) << 32) | (1ull << 46) | (4ull << 61);
-}
-// B operand (weights): K-major, no swizzle: 8-row x 16-byte core matrices; LBO = byte distance between the two 16-byte K
-// chunks of one MMA, SBO = byte distance between consecutive 8-row groups.
-__device__ __forceinline__ uint64_t make_desc_noswz(uint32_t addr, uint32_t lbo, uint32_t sbo) {
-    return (uint64_t)((addr & 0x3FFFF) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) | (1ull << 46);
-}
-
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t* r) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-                 : "r"(taddr));
-}
 
 __global__ void __launch_bounds__(C0_THREADS, 1)
 conv0_ring_kernel(const __grid_constant__ CUtensorMap tmIn, const Conv0Params p, int batch) {
@@ -142,7 +124,8 @@ conv0_ring_kernel(const __grid_constant__ CUtensorMap tmIn, const Conv0Params p,
                 ptx::mbar_wait(full_bar(stage), phase, p.err, 13);
                 ptx::tc_fence_after();
                 const uint32_t sa = smem_base + stage * C0_STAGE_BYTES;
-                const uint64_t a0 = make_desc_sw64(sa);
+                // A: 64-byte swizzled rows of 32 channels (one MMA consumes 32 B of each); B (weights): unswizzled core matrices
+                const uint64_t a0 = make_smem_desc<32>(sa);
                 const uint64_t b0 = make_desc_noswz(w_base, C0_N * 16, 128);
 #pragma unroll
                 for (int r = 0; r < C0_R + 2; ++r) {
@@ -228,7 +211,7 @@ conv0_ring_kernel(const __grid_constant__ CUtensorMap tmIn, const Conv0Params p,
 #pragma unroll
                         for (int ky = 0; ky < 3; ++ky)
                             if (rl - ky >= 0 && rl - ky < RG)
-                                tmem_ld8(lane_addr + (uint32_t)(slot * C0_N + (kz * 3 + ky) * 8), rr[kz][ky]);
+                                ptx::tmem_ld8(lane_addr + (uint32_t)(slot * C0_N + (kz * 3 + ky) * 8), rr[kz][ky]);
                     ptx::tmem_ld_wait();
                     ptx::tc_fence_before();
                     __syncwarp();
@@ -269,34 +252,21 @@ struct Conv0Plan {
     int num_sms;
 };
 
-int tc_conv_init_driver();
-extern PFN_cuTensorMapEncodeTiled_v12000 g_encode_shared;
-
 Conv0Plan* conv0_alloc() { return new Conv0Plan(); }
 void conv0_release(Conv0Plan* p) { delete p; }
 
 int conv0_plan(Conv0Plan* pl, const Act& in, const uint16_t* w_packed, const float* scale, const float* shift, uint16_t* out,
                int flags, int num_sms) {
-    const int planar = flags & 1;
-    ADP_TRY(tc_conv_init_driver());
+    ADP_TRY(tma_init_driver());
     ADP_CHECK_ARG(in.C == 32 && in.W % C0_SEG == 0 && in.D >= 2 && in.H % C0_R == 0,
                   "conv0 ring kernel: C = 32, W % 112 == 0, D >= 2, H % 4 == 0");
     // plane D-1 of an odd D would land at s2d depth (D-1)/2, one past the end of a [B, D/2, ...] output
     ADP_CHECK_ARG(!(flags & 2) || in.D % 2 == 0, "conv0 ring kernel: the space-to-depth(2) output layout needs an even D");
-    cuuint64_t dims[5] = {(cuuint64_t)in.C, (cuuint64_t)in.W, (cuuint64_t)in.H, (cuuint64_t)in.D, (cuuint64_t)in.B};
-    cuuint64_t strides[4] = {(cuuint64_t)in.C * 2, (cuuint64_t)in.W * in.C * 2, (cuuint64_t)in.H * in.W * in.C * 2,
-                             (cuuint64_t)in.D * in.H * in.W * in.C * 2};
-    cuuint32_t box[5] = {32, (cuuint32_t)C0_PIXPITCH, (cuuint32_t)(C0_R + 2), 1, 1};
-    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    ADP_CHECK_ARG(!planar, "the depth-ring kernel reads the channels-last volume");
-    const int rank = 5;
-    CUresult r = g_encode_shared(&pl->tmIn, in.f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, in.hi, dims,
-                                 strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-                                 CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_last_error("cuTensorMapEncodeTiled(conv0 volume) failed: %d", (int)r);
-        return ADP_ERR_CUDA;
-    }
+    ADP_CHECK_ARG(!(flags & 1), "the depth-ring kernel reads the channels-last volume");
+    const cuuint64_t dims[5] = {(cuuint64_t)in.C, (cuuint64_t)in.W, (cuuint64_t)in.H, (cuuint64_t)in.D, (cuuint64_t)in.B};
+    const cuuint32_t box[5] = {32, (cuuint32_t)C0_PIXPITCH, (cuuint32_t)(C0_R + 2), 1, 1};
+    ADP_TRY(tma_encode(&pl->tmIn, tma_type16(in.f16), 5, in.hi, dims, 2, box, nullptr, CU_TENSOR_MAP_SWIZZLE_64B,
+                       CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "conv0 volume"));
     pl->p.B = in.B; pl->p.D = in.D; pl->p.H = in.H; pl->p.W = in.W; pl->p.f16 = in.f16;
     pl->p.w = w_packed; pl->p.scale = scale; pl->p.shift = shift; pl->p.out = out; pl->p.err = nullptr; pl->p.out_s2d = (flags >> 1) & 1;
     pl->num_sms = num_sms > 0 ? num_sms : 148;

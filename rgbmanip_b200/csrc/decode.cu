@@ -6,8 +6,7 @@
 //   pose feature   = pose_mlp1(cat(fused, nocs_pts_mlp(NOCS)))  -> per-env mean -> pose_mlp2 -> mean -> rotation head
 // Kernels here: decode_gather (the gather / memory-bound part), colsum (deterministic per-env sums), pose_gbias, rot_head; the
 // per-point MLPs are 1x1 convolutions on the tcgen05 conv kernel (engine.py: _build_decode_tc).
-#include "../../include/adapose_b200.h"
-#include "common.cuh"
+#include "stages.cuh"
 #include "warp.cuh"
 
 namespace adp {
@@ -15,24 +14,6 @@ namespace adp {
 constexpr int PB = 32;          // sampled pixels per block
 constexpr int DEC_THREADS = 256;
 constexpr int LDS = 260;        // padded row pitch (floats) of the activation ping-pong buffers, multiple of 4
-
-struct DecodeWeights {
-    // all fp32, transposed to [K][N] so that threads read consecutive output columns
-    const float* ic_w;  const float* ic_b;      // instance_color 32 -> 64
-    const float* nh0_w; const float* nh0_b;     // nocs_head 64 -> 128
-    const float* nh1_w; const float* nh1_b;     // 128 -> 64
-    const float* nh2_w; const float* nh2_b;     // 64 -> 3
-    const float* np0_w; const float* np0_b;     // nocs_pts_mlp 3 -> 32
-    const float* np1_w; const float* np1_b;     // 32 -> 64
-    const float* pm0_w; const float* pm0_b;     // pose_mlp1 96 -> 128
-    const float* pm1_w; const float* pm1_b;     // 128 -> 128
-    const float* q0_w;  const float* q0_b;      // pose_mlp2 256 -> 256
-    const float* q1_w;  const float* q1_b;      // 256 -> 256
-    const float* r0_w;  const float* r0_b;      // rotation_estimator 256 -> 256
-    const float* r1_w;  const float* r1_b;      // 256 -> 128
-    const float* r2_w;  const float* r2_b;      // 128 -> 6
-    const float* prob_w;                        // [27][8] depth-logit conv
-};
 
 struct DecodeArgs {
     const float* feat_ref;   // [B,S,S,32] fp32
@@ -280,7 +261,7 @@ __global__ void pose_gbias_kernel(const float* __restrict__ gsum, const float* _
 // rotation head 256 -> 256 -> 128 -> 6 and the 6-D -> SO(3) map (ADA/lib/rotation_utils.py:4-27)
 __global__ void __launch_bounds__(256)
 rot_head_kernel(const float* __restrict__ psum, const uint8_t* __restrict__ valid, float* __restrict__ Rout, float* __restrict__ r6out,
-                const DecodeWeights w, int P) {
+                const adp_decode_weights w, int P) {
     __shared__ float v0[256], v1[256], v2[128], r6[6];
     const int b = blockIdx.x, tid = threadIdx.x;
     if (valid && !valid[b]) {
@@ -359,9 +340,7 @@ int pose_gbias_run(const float* gsum, const float* q0_w, const float* q0_b, cons
 int rot_head_run(const float* psum, const uint8_t* valid, float* Rout, float* r6out, const adp_decode_weights* cw, int B, int P,
                  cudaStream_t stream) {
     if (B == 0) return ADP_OK;
-    DecodeWeights w{};
-    w.r0_w = cw->r0_w; w.r0_b = cw->r0_b; w.r1_w = cw->r1_w; w.r1_b = cw->r1_b; w.r2_w = cw->r2_w; w.r2_b = cw->r2_b;
-    rot_head_kernel<<<B, 256, 0, stream>>>(psum, valid, Rout, r6out, w, P);
+    rot_head_kernel<<<B, 256, 0, stream>>>(psum, valid, Rout, r6out, *cw, P);
     ADP_CUDA(cudaGetLastError());
     return ADP_OK;
 }

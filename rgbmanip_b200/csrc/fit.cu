@@ -9,7 +9,7 @@
 // (explicitly rounded intrinsics in a fixed order, so every pass sees the same bits): ~30 instructions per pair instead of a
 // 2 MB-per-environment scratch row that is written once and re-read three times.  The per-CTA histograms are summed over distributed shared memory, so every CTA
 // of the cluster derives the same digit without a broadcast.
-#include "common.cuh"
+#include "stages.cuh"
 
 #include <cooperative_groups.h>
 

@@ -4,7 +4,7 @@
 // box construction as branch A (interface_v5.py:354-374).  One CTA per environment, everything in fp64 like numpy.
 // The 128 x 5 sample indices come either from a caller-supplied table (exact replay of a numpy stream in the parity
 // tests) or from a counter-based hash (same distribution as np.random.randint, different stream).
-#include "common.cuh"
+#include "stages.cuh"
 
 namespace adp {
 

@@ -9,7 +9,7 @@
 //   5. transform into the view-1 camera frame (left_pose @ X).
 // One CTA of 1024 threads per environment, both NOCS maps in shared memory.  The median scale of the matched set is taken by
 // the fit kernel in points mode (csrc/fit.cu); the PnP tail (cv2.solvePnPRansac) stays on the host.
-#include "common.cuh"
+#include "stages.cuh"
 
 namespace adp {
 

@@ -3,7 +3,7 @@
 //   -> bilinear crop resize to S x S (cv2 INTER_LINEAR semantics) + ImageNet normalisation
 //   -> nearest mask resize (cv2 INTER_NEAREST index rule) -> exactly P sampled foreground indices
 //   -> crop-adjusted intrinsics K'.
-#include "common.cuh"
+#include "stages.cuh"
 
 namespace adp {
 

@@ -163,9 +163,29 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* r) {
           "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
         : "r"(taddr));
 }
+__device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t* r) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+                 : "r"(taddr));
+}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 }  // namespace ptx
+
+// Shared-memory matrix descriptor, K-major operand whose rows are KC*2 bytes (= the swizzle span).
+//   [0,14) start >> 4 | [16,30) LBO >> 4 (unused for swizzled K-major) | [32,46) SBO >> 4 (8-row group pitch)
+//   [46,48) version = 1 (sm_100) | [49,52) base offset = 0 (tiles are 1024B aligned) | [61,64) layout type
+template <int KC>
+__device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
+    constexpr uint64_t layout = (KC == 64) ? 2ull : (KC == 32) ? 4ull : 6ull;   // SWIZZLE_128B / 64B / 32B
+    constexpr uint64_t sbo = (uint64_t)(8 * KC * 2) >> 4;
+    return (uint64_t)((smem_addr & 0x3FFFF) >> 4) | (1ull << 16) | (sbo << 32) | (1ull << 46) | (layout << 61);
+}
+// K-major operand without swizzle: 8-row x 16-byte core matrices; LBO = byte distance between the two 16-byte K chunks of one
+// MMA, SBO = byte distance between consecutive 8-row groups.
+__device__ __forceinline__ uint64_t make_desc_noswz(uint32_t addr, uint32_t lbo, uint32_t sbo) {
+    return (uint64_t)((addr & 0x3FFFF) >> 4) | ((uint64_t)(lbo >> 4) << 16) | ((uint64_t)(sbo >> 4) << 32) | (1ull << 46);
+}
 
 // Instruction descriptor for kind::f16: D = fp32, A = B = bf16 (or fp16), both K-major, M = 128, N = n.
 __device__ __forceinline__ uint32_t make_idesc_n(int n, int f16) {

@@ -1,30 +1,12 @@
 // tcgen05 implicit-GEMM convolution -- see tc_conv.cuh for the scheme.
 #include "tc_conv.cuh"
 #include "ptx.cuh"
+#include "tma.cuh"
 
 #include <cudaTypedefs.h>
 #include <stdlib.h>
 
 namespace adp {
-
-// ------------------------------------------------------------------------------------------------
-// descriptors
-// ------------------------------------------------------------------------------------------------
-// Shared-memory matrix descriptor, K-major operand whose rows are KC*2 bytes (= the swizzle span).
-//   [0,14) start >> 4 | [16,30) LBO >> 4 (unused for swizzled K-major) | [32,46) SBO >> 4 (8-row group pitch)
-//   [46,48) version = 1 (sm_100) | [49,52) base offset = 0 (tiles are 1024B aligned) | [61,64) layout type
-template <int KC>
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
-    constexpr uint64_t layout = (KC == 64) ? 2ull : (KC == 32) ? 4ull : 6ull;   // SWIZZLE_128B / 64B / 32B
-    constexpr uint64_t sbo = (uint64_t)(8 * KC * 2) >> 4;
-    return (uint64_t)((smem_addr & 0x3FFFF) >> 4) | (1ull << 16) | (sbo << 32) | (1ull << 46) | (layout << 61);
-}
-// Instruction descriptor for kind::f16: D = fp32, A = B = bf16, both K-major, M = 128, N = BN.
-template <int BN>
-__device__ __forceinline__ uint32_t make_idesc(int f16) {
-    const uint32_t fmt = f16 ? 0u : 1u;   // F16 = 0, BF16 = 1
-    return (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-}
 
 // ------------------------------------------------------------------------------------------------
 // kernel
@@ -465,7 +447,7 @@ tc_conv_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
         uint32_t phase = 0;
         int as = 0;
         uint32_t aphase = 0;
-        const uint32_t idesc = make_idesc<BN>(p.f16);
+        const uint32_t idesc = make_idesc_n(BN, p.f16);
         const uint32_t elected = ptx::elect_one();
         const uint32_t tbase = __shfl_sync(0xffffffffu, tmem_base, 0);
         for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
@@ -736,7 +718,7 @@ slab_conv_kernel(const __grid_constant__ CUtensorMap tmSlab, const __grid_consta
         // ===================== MMA issuer (warp-convergent, elected lane) =====================
         int stage = 0, as = 0;
         uint32_t phase = 0, aphase = 0;
-        const uint32_t idesc = make_idesc<BN>(p.f16);
+        const uint32_t idesc = make_idesc_n(BN, p.f16);
         const uint32_t elected = ptx::elect_one();
         const uint32_t tbase = __shfl_sync(0xffffffffu, tmem_base, 0);
         const uint32_t sbo = (uint32_t)(p.sSX * KC * 2);
@@ -887,9 +869,8 @@ slab_conv_kernel(const __grid_constant__ CUtensorMap tmSlab, const __grid_consta
 // host side
 // ------------------------------------------------------------------------------------------------
 static PFN_cuTensorMapEncodeTiled_v12000 g_encode = nullptr;
-PFN_cuTensorMapEncodeTiled_v12000 g_encode_shared = nullptr;   // for the other tcgen05 translation units
 
-int tc_conv_init_driver() {
+int tma_init_driver() {
     if (g_encode) return ADP_OK;
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult qres;
@@ -899,7 +880,26 @@ int tc_conv_init_driver() {
         return ADP_ERR_CUDA;
     }
     g_encode = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
-    g_encode_shared = g_encode;
+    return ADP_OK;
+}
+
+int tma_encode(CUtensorMap* tm, CUtensorMapDataType dt, int rank, const void* ptr, const cuuint64_t* dims, int esize,
+               const cuuint32_t* box, const cuuint32_t* estr, CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2,
+               const char* what) {
+    ADP_CHECK_ARG(rank >= 1 && rank <= 5, "tensor map rank");
+    cuuint64_t strides[4];
+    const cuuint32_t ones[5] = {1, 1, 1, 1, 1};
+    for (int i = 0; i + 1 < rank; ++i) strides[i] = (i ? strides[i - 1] : (cuuint64_t)esize) * dims[i];
+    const CUresult r = g_encode(tm, dt, rank, const_cast<void*>(ptr), dims, strides, box, estr ? estr : ones,
+                                CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        char shape[256];   // <= 5 x 34 characters
+        int n = 0;
+        for (int i = 0; i < rank; ++i)
+            n += snprintf(shape + n, sizeof(shape) - n, "%s%llu/%u", i ? " x " : "", (unsigned long long)dims[i], box[i]);
+        set_last_error("cuTensorMapEncodeTiled(%s: dims/box %s) failed: %d", what, shape, (int)r);
+        return ADP_ERR_CUDA;
+    }
     return ADP_OK;
 }
 
@@ -910,39 +910,19 @@ static CUtensorMapSwizzle swizzle_for(int KC) {
 // esize 2: 16-bit plane (f16 selects half / bf16), KC channels per box; esize 1: the fp8 twin, 128 one-byte channels per box (the
 // rows are 128 bytes either way -> SWIZZLE_128B)
 static int encode_act_map(CUtensorMap* tm, const void* ptr, const Act& a, int KC, int TW, int TH, int in_mul, int f16, int esize = 2) {
-    cuuint64_t dims[5] = {(cuuint64_t)a.C, (cuuint64_t)a.W, (cuuint64_t)a.H, (cuuint64_t)a.D, (cuuint64_t)a.B};
-    cuuint64_t strides[4] = {(cuuint64_t)a.C * esize, (cuuint64_t)a.W * a.C * esize, (cuuint64_t)a.H * a.W * a.C * esize,
-                             (cuuint64_t)a.D * a.H * a.W * a.C * esize};
+    const cuuint64_t dims[5] = {(cuuint64_t)a.C, (cuuint64_t)a.W, (cuuint64_t)a.H, (cuuint64_t)a.D, (cuuint64_t)a.B};
     // with an element stride s the unit loads ceil(box / s) elements: a box of (T-1)*s+1 yields exactly T
-    cuuint32_t box[5] = {(cuuint32_t)KC, (cuuint32_t)((TW - 1) * in_mul + 1), (cuuint32_t)((TH - 1) * in_mul + 1), 1, 1};
-    cuuint32_t estr[5] = {1, (cuuint32_t)in_mul, (cuuint32_t)in_mul, (cuuint32_t)(a.D > 1 ? in_mul : 1), 1};
-    const CUtensorMapDataType dt = esize == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-    CUresult r = g_encode(tm, dt, 5, const_cast<void*>(ptr), dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, esize == 1 ? CU_TENSOR_MAP_SWIZZLE_128B : swizzle_for(KC), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_last_error("cuTensorMapEncodeTiled(activation C=%d W=%d H=%d D=%d B=%d box=%dx%dx%d) failed: %d", a.C, a.W, a.H,
-                       a.D, a.B, KC, TW, TH, (int)r);
-        return ADP_ERR_CUDA;
-    }
-    return ADP_OK;
+    const cuuint32_t box[5] = {(cuuint32_t)KC, (cuuint32_t)((TW - 1) * in_mul + 1), (cuuint32_t)((TH - 1) * in_mul + 1), 1, 1};
+    const cuuint32_t estr[5] = {1, (cuuint32_t)in_mul, (cuuint32_t)in_mul, (cuuint32_t)(a.D > 1 ? in_mul : 1), 1};
+    return tma_encode(tm, esize == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : tma_type16(f16), 5, ptr, dims, esize, box, estr,
+                      esize == 1 ? CU_TENSOR_MAP_SWIZZLE_128B : swizzle_for(KC), CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "activation");
 }
 
 static int encode_w_map(CUtensorMap* tm, const void* ptr, int Cin, int CoutPad, int taps, int KC, int BN, int f16, int esize = 2) {
-    cuuint64_t dims[3] = {(cuuint64_t)Cin, (cuuint64_t)CoutPad, (cuuint64_t)taps};
-    cuuint64_t strides[2] = {(cuuint64_t)Cin * esize, (cuuint64_t)CoutPad * Cin * esize};
-    cuuint32_t box[3] = {(cuuint32_t)KC, (cuuint32_t)BN, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    const CUtensorMapDataType dt = esize == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-    CUresult r = g_encode(tm, dt, 3, const_cast<void*>(ptr), dims, strides, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, esize == 1 ? CU_TENSOR_MAP_SWIZZLE_128B : swizzle_for(KC), CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_last_error("cuTensorMapEncodeTiled(weights Cin=%d Cout=%d taps=%d box=%dx%d) failed: %d", Cin, CoutPad, taps, KC,
-                       BN, (int)r);
-        return ADP_ERR_CUDA;
-    }
-    return ADP_OK;
+    const cuuint64_t dims[3] = {(cuuint64_t)Cin, (cuuint64_t)CoutPad, (cuuint64_t)taps};
+    const cuuint32_t box[3] = {(cuuint32_t)KC, (cuuint32_t)BN, 1};
+    return tma_encode(tm, esize == 1 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : tma_type16(f16), 3, ptr, dims, esize, box, nullptr,
+                      esize == 1 ? CU_TENSOR_MAP_SWIZZLE_128B : swizzle_for(KC), CU_TENSOR_MAP_L2_PROMOTION_L2_256B, "weights");
 }
 
 void tc_pick_tile(int H, int W, int* TW, int* TH) {
@@ -964,8 +944,8 @@ void tc_pick_tile(int H, int W, int* TW, int* TH) {
 }
 
 int tc_conv_plan(TcConvLayer* L, const Act& in, const bf16* w_hi, const bf16* w_lo, int Cout, int kd, int ks, int dil,
-                 int npass, const TcGeom* geom, int f16) {
-    ADP_TRY(tc_conv_init_driver());
+                 int npass, const adp_tc_geom* geom, int f16) {
+    ADP_TRY(tma_init_driver());
     int KC = in.C % 64 == 0 ? 64 : in.C % 32 == 0 ? 32 : in.C % 16 == 0 ? 16 : 0;
     ADP_CHECK_ARG(KC != 0, "Cin must be a multiple of 16 for the tcgen05 path");
     ADP_CHECK_ARG(npass >= 1 && npass <= 4, "npass");
@@ -1041,18 +1021,10 @@ int tc_conv_plan(TcConvLayer* L, const Act& in, const bf16* w_hi, const bf16* w_
             if (stages >= 2) {
                 p.slab_stages = stages;
                 L->slab_ctas = ctas;
-                cuuint64_t dims[5] = {(cuuint64_t)in.C, (cuuint64_t)in.W, (cuuint64_t)in.H, (cuuint64_t)in.D, (cuuint64_t)in.B};
-                cuuint64_t strides[4] = {(cuuint64_t)in.C * 2, (cuuint64_t)in.W * in.C * 2, (cuuint64_t)in.H * in.W * in.C * 2,
-                                         (cuuint64_t)in.D * in.H * in.W * in.C * 2};
-                cuuint32_t box[5] = {(cuuint32_t)KC, (cuuint32_t)p.sSX, (cuuint32_t)p.sSY, (cuuint32_t)p.sSZ, 1};
-                cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-                CUresult r = g_encode(&L->tmSlab, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, in.hi, dims,
-                                      strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_for(KC), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-                if (r != CUDA_SUCCESS) {
-                    set_last_error("cuTensorMapEncodeTiled(slab %dx%dx%d x %d) failed: %d", p.sSX, p.sSY, p.sSZ, KC, (int)r);
-                    return ADP_ERR_CUDA;
-                }
+                const cuuint64_t dims[5] = {(cuuint64_t)in.C, (cuuint64_t)in.W, (cuuint64_t)in.H, (cuuint64_t)in.D, (cuuint64_t)in.B};
+                const cuuint32_t box[5] = {(cuuint32_t)KC, (cuuint32_t)p.sSX, (cuuint32_t)p.sSY, (cuuint32_t)p.sSZ, 1};
+                ADP_TRY(tma_encode(&L->tmSlab, tma_type16(f16), 5, in.hi, dims, 2, box, nullptr, swizzle_for(KC),
+                                   CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "slab"));
             } else {
                 tc_pick_tile(p.H, p.W, &p.TW, &p.TH);
                 p.tiles_x = cdiv(p.W, p.TW); p.tiles_y = cdiv(p.H, p.TH);
@@ -1087,20 +1059,12 @@ static int tc_conv_pick_bulk_epilogue(TcConvLayer* L) {
     int stages = p.slab_stages;
     while (stages >= 2 && stages * stage_bytes + fixed > 111 * 1024) --stages;
     if (stages < 2) return ADP_OK;
-    cuuint64_t dims[5] = {64, (cuuint64_t)p.oW, (cuuint64_t)p.oH, (cuuint64_t)p.oD, (cuuint64_t)p.B};
-    cuuint64_t strides[4] = {128, (cuuint64_t)p.oW * 128, (cuuint64_t)p.oH * p.oW * 128, (cuuint64_t)p.oD * p.oH * p.oW * 128};
-    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    cuuint32_t box_r[5] = {64, 8, 16, 1, 1}, box_o[5] = {64, 8, 4, 1, 1};
-    CUresult r = g_encode(&L->tmRes, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, const_cast<bf16*>(p.res_hi), dims, strides, box_r, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r == CUDA_SUCCESS)
-        r = g_encode(&L->tmOut, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, p.out_hi, dims, strides, box_o, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-        set_last_error("cuTensorMapEncodeTiled(residual / output tiles %dx%dx%d) failed: %d", p.oW, p.oH, p.oD, (int)r);
-        return ADP_ERR_CUDA;
-    }
+    const cuuint64_t dims[5] = {64, (cuuint64_t)p.oW, (cuuint64_t)p.oH, (cuuint64_t)p.oD, (cuuint64_t)p.B};
+    const cuuint32_t box_r[5] = {64, 8, 16, 1, 1}, box_o[5] = {64, 8, 4, 1, 1};
+    ADP_TRY(tma_encode(&L->tmRes, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, p.res_hi, dims, 2, box_r, nullptr, CU_TENSOR_MAP_SWIZZLE_128B,
+                       CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "residual tiles"));
+    ADP_TRY(tma_encode(&L->tmOut, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 5, p.out_hi, dims, 2, box_o, nullptr, CU_TENSOR_MAP_SWIZZLE_128B,
+                       CU_TENSOR_MAP_L2_PROMOTION_L2_128B, "output tiles"));
     p.slab_stages = stages;
     L->bulk_epi = true;
     return ADP_OK;

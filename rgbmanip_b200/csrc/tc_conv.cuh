@@ -13,6 +13,7 @@
 // three passes (A_hi W_hi, A_lo W_hi, A_hi W_lo) into the same fp32 accumulator, which restores ~16
 // mantissa bits -- see DESIGN.md "precision policy".
 #pragma once
+#include "../../include/adapose_b200.h"
 #include "common.cuh"
 
 namespace adp {
@@ -75,19 +76,11 @@ struct TcConvLayer {
     int instance = -1;       // its row in the instance table of tc_conv.cu (reported by tc_conv_plan_info)
 };
 
-int tc_conv_init_driver();
-struct TcGeom {             // non-standard geometries (NULL = stride-1 "same" conv with a kd x ks x ks window)
-    int ntaps;
-    signed char dz[32], dy[32], dx[32], wt[32];
-    int in_mul;
-    int out_mul, out_oz, out_oy, out_ox;
-    int gD, gH, gW;
-    int oD, oH, oW;
-    int w_taps;             // number of tap slabs in the packed weight tensor
-};
-
+// a rectangle of <= 128 output pixels for an H x W map (also the tile of the fused transposed conv)
+void tc_pick_tile(int H, int W, int* TW, int* TH);
+// geom: non-standard geometry (NULL = stride-1 "same" conv with a kd x ks x ks window)
 int tc_conv_plan(TcConvLayer* L, const Act& in, const bf16* w_hi, const bf16* w_lo, int Cout, int kd, int ks,
-                 int dil, int npass, const TcGeom* geom, int f16);
+                 int dil, int npass, const adp_tc_geom* geom, int f16);
 // after the epilogue fields of L->p are set: picks the TMA epilogue where it applies and the kernel instance; ADP_ERR_ARG when
 // the library has no instance for the layer's tile, K step and pass mode
 int tc_conv_finish_plan(TcConvLayer* L);

@@ -7,10 +7,10 @@
 // (8, 4, 4, 2, 4, 2, 2, 1 of them) into that class's own 16/32-column TMEM region; the weights of all 27 taps stay
 // resident in shared memory.  Compared with 8 separate class launches the input is fetched 8x instead of 27x per
 // tile and a tile amortises its pipeline latency over 27 MMAs and 8 output voxels per input position.
-#include "common.cuh"
 #include "ptx.cuh"
-
-#include <cudaTypedefs.h>
+#include "stages.cuh"
+#include "tc_conv.cuh"
+#include "tma.cuh"
 
 namespace adp {
 
@@ -29,13 +29,6 @@ struct TconvParams {
     bf16* out;               // [B, 2D, 2H, 2W, Cout]
     int* err;
 };
-
-template <int KC>
-__device__ __forceinline__ uint64_t tf_smem_desc(uint32_t smem_addr) {
-    constexpr uint64_t layout = (KC == 64) ? 2ull : (KC == 32) ? 4ull : 6ull;
-    constexpr uint64_t sbo = (uint64_t)(8 * KC * 2) >> 4;
-    return (uint64_t)((smem_addr & 0x3FFFF) >> 4) | (1ull << 16) | (sbo << 32) | (1ull << 46) | (layout << 61);
-}
 
 template <int KC, int BN>
 struct TfCfg {
@@ -125,7 +118,7 @@ tconv_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                 ptx::mbar_wait(full_bar(stage), phase, p.err, 24);
                 ptx::tc_fence_after();
                 {
-                    const uint64_t adesc = tf_smem_desc<KC>(smem_base + stage * Cfg::A_BYTES);
+                    const uint64_t adesc = make_smem_desc<KC>(smem_base + stage * Cfg::A_BYTES);
                     const int oz = o >> 2, oy = (o >> 1) & 1, ox = o & 1;
                     // per axis: offset 0 serves (parity 0, k = 1) and (parity 1, k = 2); offset 1 serves (parity 1, k = 0)
                     for (int cz = 0; cz < (oz ? 1 : 2); ++cz)
@@ -134,7 +127,7 @@ tconv_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                                 const int pz = oz ? 1 : cz, py = oy ? 1 : cy, px = ox ? 1 : cx;
                                 const int kz = oz ? 0 : (pz ? 2 : 1), ky = oy ? 0 : (py ? 2 : 1), kx = ox ? 0 : (px ? 2 : 1);
                                 const int cls = (pz << 2) | (py << 1) | px, tap = (kz * 3 + ky) * 3 + kx;
-                                const uint64_t bdesc = tf_smem_desc<KC>(w_base + tap * Cfg::W_SLOT);
+                                const uint64_t bdesc = make_smem_desc<KC>(w_base + tap * Cfg::W_SLOT);
                                 const uint32_t tmem_d = tmem_set + (uint32_t)(cls * Cfg::REGION);
 #pragma unroll
                                 for (int k = 0; k < KC / 16; ++k)
@@ -212,56 +205,12 @@ tconv_fused_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
 struct TconvPlan {
     CUtensorMap tmA, tmW;
     TconvParams p;
-    int KC, BN, num_sms;
+    int num_sms;
+    int (*launch)(const TconvPlan* pl, int batch, cudaStream_t stream);   // the kernel instance of (KC, BN), chosen by tconv_plan
 };
 
-int tc_conv_init_driver();
-extern PFN_cuTensorMapEncodeTiled_v12000 g_encode_shared;
-void tc_pick_tile(int H, int W, int* TW, int* TH);
-
-TconvPlan* tconv_alloc() { return new TconvPlan(); }
-void tconv_release(TconvPlan* p) { delete p; }
-
-int tconv_plan(TconvPlan* pl, const Act& in, const bf16* w, int Cout, const float* scale, const float* bias, const bf16* res,
-               int res_cs, bf16* out, int flags, int num_sms) {
-    ADP_TRY(tc_conv_init_driver());
-    ADP_CHECK_ARG((in.C == 16 || in.C == 32) && Cout % 8 == 0 && Cout <= 32, "fused transposed conv: Cin in {16,32}, Cout in {8,16,32}");
-    ADP_CHECK_ARG(in.lo == nullptr, "single-plane activations only");
-    const int KC = in.C;
-    const int BN = Cout <= 16 ? 16 : 32;
-    TconvParams& p = pl->p;
-    p = TconvParams{};
-    p.B = in.B; p.D = in.D; p.H = in.H; p.W = in.W; p.Cout = Cout; p.res_cs = res_cs ? res_cs : Cout; p.f16 = in.f16; p.s2d = (flags >> 1) & 1;
-    tc_pick_tile(in.H, in.W, &p.TW, &p.TH);
-    p.tiles_x = cdiv(in.W, p.TW); p.tiles_y = cdiv(in.H, p.TH);
-    p.scale = scale; p.bias = bias; p.res = res; p.out = out; p.err = nullptr;
-    const CUtensorMapSwizzle swz = KC == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
-    const CUtensorMapDataType dt = in.f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-    {
-        cuuint64_t dims[5] = {(cuuint64_t)in.C, (cuuint64_t)in.W, (cuuint64_t)in.H, (cuuint64_t)in.D, (cuuint64_t)in.B};
-        cuuint64_t strides[4] = {(cuuint64_t)in.C * 2, (cuuint64_t)in.W * in.C * 2, (cuuint64_t)in.H * in.W * in.C * 2,
-                                 (cuuint64_t)in.D * in.H * in.W * in.C * 2};
-        cuuint32_t box[5] = {(cuuint32_t)KC, (cuuint32_t)p.TW, (cuuint32_t)p.TH, 1, 1};
-        cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-        CUresult r = g_encode_shared(&pl->tmA, dt, 5, in.hi, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
-                                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { set_last_error("cuTensorMapEncodeTiled(tconv input) failed: %d", (int)r); return ADP_ERR_CUDA; }
-    }
-    {
-        cuuint64_t dims[3] = {(cuuint64_t)in.C, (cuuint64_t)BN, 27};
-        cuuint64_t strides[2] = {(cuuint64_t)in.C * 2, (cuuint64_t)BN * in.C * 2};
-        cuuint32_t box[3] = {(cuuint32_t)KC, (cuuint32_t)BN, 1};
-        cuuint32_t estr[3] = {1, 1, 1};
-        CUresult r = g_encode_shared(&pl->tmW, dt, 3, const_cast<bf16*>(w), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
-                                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { set_last_error("cuTensorMapEncodeTiled(tconv weights) failed: %d", (int)r); return ADP_ERR_CUDA; }
-    }
-    pl->KC = KC; pl->BN = BN; pl->num_sms = num_sms > 0 ? num_sms : 148;
-    return ADP_OK;
-}
-
 template <int KC, int BN>
-static int tconv_launch(TconvPlan* pl, int batch, cudaStream_t stream) {
+static int tconv_launch(const TconvPlan* pl, int batch, cudaStream_t stream) {
     using Cfg = TfCfg<KC, BN>;
     static int attr[kMaxDevices];
     ADP_TRY(ensure_dyn_smem(tconv_fused_kernel<KC, BN>, Cfg::SMEM, attr));
@@ -274,15 +223,47 @@ static int tconv_launch(TconvPlan* pl, int batch, cudaStream_t stream) {
     return ADP_OK;
 }
 
+TconvPlan* tconv_alloc() { return new TconvPlan(); }
+void tconv_release(TconvPlan* p) { delete p; }
+
+int tconv_plan(TconvPlan* pl, const Act& in, const bf16* w, int Cout, const float* scale, const float* bias, const bf16* res,
+               int res_cs, bf16* out, int flags, int num_sms) {
+    ADP_TRY(tma_init_driver());
+    ADP_CHECK_ARG((in.C == 16 || in.C == 32) && Cout % 8 == 0 && Cout <= 32, "fused transposed conv: Cin in {16,32}, Cout in {8,16,32}");
+    ADP_CHECK_ARG(in.lo == nullptr, "single-plane activations only");
+    const int KC = in.C;
+    const int BN = Cout <= 16 ? 16 : 32;
+    TconvParams& p = pl->p;
+    p = TconvParams{};
+    p.B = in.B; p.D = in.D; p.H = in.H; p.W = in.W; p.Cout = Cout; p.res_cs = res_cs ? res_cs : Cout; p.f16 = in.f16; p.s2d = (flags >> 1) & 1;
+    tc_pick_tile(in.H, in.W, &p.TW, &p.TH);
+    p.tiles_x = cdiv(in.W, p.TW); p.tiles_y = cdiv(in.H, p.TH);
+    p.scale = scale; p.bias = bias; p.res = res; p.out = out; p.err = nullptr;
+    const CUtensorMapSwizzle swz = KC == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
+    const cuuint64_t dims_a[5] = {(cuuint64_t)in.C, (cuuint64_t)in.W, (cuuint64_t)in.H, (cuuint64_t)in.D, (cuuint64_t)in.B};
+    const cuuint32_t box_a[5] = {(cuuint32_t)KC, (cuuint32_t)p.TW, (cuuint32_t)p.TH, 1, 1};
+    ADP_TRY(tma_encode(&pl->tmA, tma_type16(in.f16), 5, in.hi, dims_a, 2, box_a, nullptr, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                       "tconv input"));
+    const cuuint64_t dims_w[3] = {(cuuint64_t)in.C, (cuuint64_t)BN, 27};
+    const cuuint32_t box_w[3] = {(cuuint32_t)KC, (cuuint32_t)BN, 1};
+    ADP_TRY(tma_encode(&pl->tmW, tma_type16(in.f16), 3, w, dims_w, 2, box_w, nullptr, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                       "tconv weights"));
+    static const struct { int KC, BN; decltype(TconvPlan::launch) launch; } instances[] = {
+        {16, 16, tconv_launch<16, 16>}, {32, 16, tconv_launch<32, 16>}, {32, 32, tconv_launch<32, 32>}, {16, 32, tconv_launch<16, 32>}};
+    pl->launch = nullptr;
+    for (const auto& t : instances) if (t.KC == KC && t.BN == BN) pl->launch = t.launch;
+    if (!pl->launch) {
+        set_last_error("no fused transposed-conv instantiation for KC=%d BN=%d", KC, BN);
+        return ADP_ERR_ARG;
+    }
+    pl->num_sms = num_sms > 0 ? num_sms : 148;
+    return ADP_OK;
+}
+
 int tconv_run(TconvPlan* pl, int batch, int* err_flag, cudaStream_t stream) {
     ADP_CHECK_ARG(batch <= pl->p.B, "batch exceeds planned capacity");
     pl->p.err = err_flag;
-    if (pl->KC == 16 && pl->BN == 16) return tconv_launch<16, 16>(pl, batch, stream);
-    if (pl->KC == 32 && pl->BN == 16) return tconv_launch<32, 16>(pl, batch, stream);
-    if (pl->KC == 32 && pl->BN == 32) return tconv_launch<32, 32>(pl, batch, stream);
-    if (pl->KC == 16 && pl->BN == 32) return tconv_launch<16, 32>(pl, batch, stream);
-    set_last_error("no fused transposed-conv instantiation for KC=%d BN=%d", pl->KC, pl->BN);
-    return ADP_ERR_ARG;
+    return pl->launch(pl, batch, stream);
 }
 
 }  // namespace adp

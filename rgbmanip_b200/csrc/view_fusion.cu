@@ -12,7 +12,7 @@
 // is fp32 on the CUDA cores: d_k = 8 is half a tensor-core K step, and at 1.1 GFLOP per environment this stage is ~1 % of the
 // network.  The last block writes the view-1 tokens as the bf16 hi/lo planes the pose MLP reads (columns 0..31 of xcat) and
 // evaluates the depth MLP (32 -> 64 -> 32 -> 1, ReLU) in the same thread.
-#include "common.cuh"
+#include "stages.cuh"
 
 namespace adp {
 

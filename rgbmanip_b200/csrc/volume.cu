@@ -3,7 +3,7 @@
 //   vol[b, d, y, x, :] = feat_ref[b, y, x, :] + bilinear(feat_src[b], u(d, y, x), v(d, y, x))
 // The coordinate convention is reproduced as written: normalise with (W-1)/2, sample with
 // align_corners=False, zeros padding.
-#include "common.cuh"
+#include "stages.cuh"
 #include "warp.cuh"
 
 namespace adp {
